@@ -2,7 +2,7 @@
 """bench.py -- interior-point iterations/s and KKT-solve ms at n = 64M (BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--config C3] [--n NTOTAL]
+                    [--config C3] [--n NTOTAL] [--dump-outputs DIR]
 
 A "step" is one pass of the interior-point major loop (IP.cpp:4607-5329) on the
 named synthetic workload (default: configs[2] of BASELINE.json -- multi-material
@@ -16,6 +16,12 @@ reference compiled in oracle/_ref, timed on a bounded sample on the host cores),
 `e2e` (same metric through the host-callback API: the iterate goes device->host
 and the gradients host->device through pinned buffers on every callback),
 `kkt_solve_ms`, `iter_roofline_frac`, `clocks`, `gpu_launches`.
+
+--dump-outputs DIR writes the optimizer's point after the last timed step as
+DIR/<name>.npy (float64): x, zl, zu, zw, sw, tw (at DUMP_SAMPLE sorted indices drawn
+with a fixed seed when longer) and the dense z, s, t, zs, zt, c.  The
+workloads are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 import argparse
 import json
@@ -28,6 +34,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from
 # stdout carries exactly one JSON line: libraries that write to file descriptor 1
 # (NCCL prints its version banner there) are sent to stderr, the line goes to the
 # saved descriptor
@@ -166,6 +173,33 @@ def iteration_words(N, W, c, q):
 
 def kkt_words(N, W, c, q):
     return (51 + 5 * c + 3 * q) * N + 62 * W
+
+
+# ------------------------------------------------------------------ outputs
+DUMP_SAMPLE = 1 << 20  # entries kept per vector: six vectors stay below 64 MB in float64
+
+
+def dump_outputs(ip, outdir):
+    """Writes the optimizer's current point (getOptimizedPoint / getOptimizedSlacks)
+    as outdir/<name>.npy, float64 (see the module docstring)."""
+    import ctypes as C
+
+    import numpy as np
+    from paropt_b200.api import PVec
+
+    os.makedirs(outdir, exist_ok=True)
+    handles = [C.c_void_p() for _ in range(6)]
+    ip.lib.pcu_ip_get_point(ip.h, *[C.byref(h) for h in handles])
+    arrays = ip.get_dense()
+    for name, h in zip(("x", "zw", "zl", "zu", "sw", "tw"), handles):
+        if not h.value:
+            continue
+        a = PVec(ip.ctx, handle=h.value).to_numpy()
+        if a.size > DUMP_SAMPLE:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        arrays[name] = a
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 # ---------------------------------------------------------------- reference
@@ -320,12 +354,29 @@ def reference_rate(cfg_name, ntotal, warmup, steps, budget_s=25.0):
 
 
 # --------------------------------------------------------------------- ours
+def iterate_exactly(ip, n):
+    """Runs n major iterations.  The default workload converges after ~96 iterations; a
+    run that converges first starts over from its starting point (begin), so that n is
+    always the number of steps.  Returns (iterations run, restarts)."""
+    done = restarts = 0
+    while True:
+        k0 = ip.counters()[0]
+        converged = ip.iterate(n - done)
+        done += ip.counters()[0] - k0
+        if done >= n or not converged:
+            return done, restarts
+        ip.begin()
+        restarts += 1
+
+
 def run_ours(args):
     import torch
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("bench: --dump-outputs writes the point of one process; use --gpus 1")
     dist = None
     if world > 1:
         import torch.distributed as dist
@@ -402,7 +453,7 @@ def run_ours(args):
     opts = dict(cfg["options"], max_major_iters=1000000, history_level=1)
     ip = InteriorPoint(prob, opts)
     ip.begin()
-    ip.iterate(warmup)
+    iterate_exactly(ip, warmup)
     barrier()
     sampler = ClockSampler(local_rank)
     if rank == 0:
@@ -416,16 +467,16 @@ def run_ours(args):
     if events_in_timed:
         ctx.profile(2)
     launches0 = ctx.kernel_launches()
-    it0 = ip.counters()[0]
     ctx.timer_start()
-    ip.iterate(steps)
+    done, restarts = iterate_exactly(ip, steps)
     ms = ctx.timer_stop()
     barrier()
     ctx.profile(0)
     clocks = sampler.stop() if rank == 0 else None
-    done = ip.counters()[0] - it0
     launches = ctx.kernel_launches() - launches0
     times = ip.iter_times()[-done:] if done else []
+    if args.dump_outputs:
+        dump_outputs(ip, args.dump_outputs)
     prof_ms = None
     if not args.no_kernel_profile and not events_in_timed:
         barrier()  # rank 0 has just joined its clock sampler
@@ -569,7 +620,7 @@ def run_ours(args):
     if rank == 0:
         line = {
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world,
-            "steps": done, "warmup": warmup, "ms_per_step": ms_per_step,
+            "steps": done, "restarts": restarts, "warmup": warmup, "ms_per_step": ms_per_step,
             "higher_is_better": True, "scaling": "weak" if weak else "strong",
             "vs_baseline": None,
             "dtype": "f64", "data": "synthetic",
@@ -637,7 +688,8 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed interior-point iterations (a run that converges restarts)")
     ap.add_argument("--warmup", type=int, default=QN_WARMUP)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="C3")
@@ -655,7 +707,11 @@ def main():
     ap.add_argument("--ref-sample", action="store_true",
                     help="--impl reference on a bounded smaller-n sample (scaled by n) "
                          "instead of the full size")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the optimizer's point after the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -85,7 +85,8 @@ def test_wide_gram_partition_covers_the_tile_triangle_once():
 
 def test_library_is_sm100a_only():
     from paropt_b200 import build
-    out = subprocess.run(["cuobjdump", "-lelf", build.LIB], capture_output=True, text=True).stdout
+    cuobjdump = os.path.join(os.path.dirname(build.NVCC), "cuobjdump")  # the toolkit that built it
+    out = subprocess.run([cuobjdump, "-lelf", build.LIB], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_\d+a?", out))
     assert archs == {"sm_100a"}, archs
 
@@ -224,7 +225,8 @@ def test_adapter_driver_links_against_the_product_library():
     resolves the C-ABI symbols the adapters call -- no compute here (no GPU)."""
     drv = os.path.join(ROOT, "oracle", "_ref", "adapter_driver")
     if not os.path.exists(drv):
-        pytest.skip("adapter_driver not built (needs /root/reference at build time)")
+        pytest.skip("adapter_driver not built (build() needs PAROPT_REF = the upstream ParOpt "
+                    "sources)")
     out = subprocess.run(["ldd", drv], capture_output=True, text=True).stdout
     assert "libparopt_b200.so" in out and "not found" not in out, out
     syms = subprocess.run(["nm", "-D", "--undefined-only", drv], capture_output=True,

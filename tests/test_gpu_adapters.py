@@ -1,6 +1,6 @@
 """The drop-in boundary, compiled and run: the UNMODIFIED reference
-ParOptInteriorPoint (objects of oracle/_ref, built from /root/reference/src where
-they lie) drives the adapter classes of tests/adapters/paropt_cuda_adapters.h --
+ParOptInteriorPoint (objects of oracle/_ref, built from the upstream ParOpt sources
+that PAROPT_REF names) drives the adapter classes of tests/adapters/paropt_cuda_adapters.h --
 ParOptCudaVec : ParOptVec, ParOptCudaQuasiDefBlockMat : ParOptQuasiDefMat,
 ParOptCudaCompactQN : ParOptCompactQuasiNewton -- injected through the reference's
 own factories (createDesignVec / createConstraintVec / createQuasiDefMat,
@@ -46,7 +46,8 @@ def run_adapter_driver(cfg, tmp_path):
                                         ("C3_nb2_small", 39), ("S1_small", None)])
 def test_reference_interior_point_runs_on_cuda_vectors(tmp_path, name, iters):
     if not os.path.exists(DRIVER):
-        pytest.skip("oracle/_ref/adapter_driver not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/adapter_driver not built (build() needs PAROPT_REF = the "
+                    "upstream ParOpt sources)")
     gold = load_golden(name)
     cfg = gold["config"]
     if iters is not None:
