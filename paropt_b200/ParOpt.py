@@ -11,11 +11,22 @@ takes a `Context` (one per GPU / rank); `ParOpt.Problem(None, ...)` opens GPU 0.
 
 `algorithm = "ip"` and `algorithm = "tr"` (SL1QP trust region, penalty method) are built;
 the MMA front end is not.
+
+`Problem` callbacks see numpy views of host mirrors: the iterate and the gradients
+cross PCIe on every call.  A problem already written in torch subclasses
+`TorchProblem` instead: the same callbacks on float64 CUDA tensors that view the
+optimizer's own device memory, run on the optimizer's stream, with no host copies
+but the objective and constraint values.  `AutogradProblem` needs only `objcon(x)
+-> (f, c)` in torch and takes the gradients and Hessian-vector products
+(`use_hvec_product`) from autograd.
+
+    class Model(ParOpt.TorchProblem):
+        def evalObjConGradient(self, x, g, A): g.copy_(...); A[0].copy_(...)
 """
 import numpy as np
 
 from . import api
-from .api import Context, PVec, QuasiDefBlockMat  # noqa: F401  (re-exported)
+from .api import AutogradProblem, Context, PVec, QuasiDefBlockMat, TorchProblem  # noqa: F401
 
 # ParOptQuasiNewton.h:18-30 enumerations, by the option strings the library takes
 SKIP_NEGATIVE_CURVATURE = "skip_negative_curvature"

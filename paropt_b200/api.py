@@ -34,7 +34,31 @@ class Context:
             raise RuntimeError(
                 "paropt_b200: could not create a CUDA context on device %d; the "
                 "interior-point core has no CPU fallback" % device)
+        self.device = int(device)
         self.rank, self.size = 0, 1
+        self._stream = None
+
+    @property
+    def stream(self):
+        """The context's CUDA stream (pcu_ctx_stream) as a torch.cuda.ExternalStream:
+        torch work enqueued there is ordered with the library's kernels."""
+        if self._stream is None:
+            import torch
+            self._stream = torch.cuda.ExternalStream(
+                int(self.lib.pcu_ctx_stream(self.h)), device=torch.device("cuda", self.device))
+        return self._stream
+
+    def allreduce_sum(self, values):
+        """Sum of `values` (host numbers, or a tensor) over the ranks of the context
+        (pcu_ctx_allreduce_sum; MPI_Allreduce(MPI_SUM) in the reference's examples),
+        as a float64 numpy array."""
+        if hasattr(values, "detach"):
+            values = values.detach().cpu().numpy()
+        out = np.array(values, dtype=np.float64).ravel()
+        if out.size:
+            _check(self.lib.pcu_ctx_allreduce_sum(self.h, out.ctypes.data_as(_lib.c_double_p),
+                                                  out.size), "allreduce_sum")
+        return out
 
     def init_distributed(self):
         """Bootstraps the NCCL communicator of this context from an initialised
@@ -507,6 +531,282 @@ class Problem:
             self.h = None
 
 
+class _DeviceArray:
+    """A library-owned device range in the CUDA array interface (no stream key: the
+    callbacks order the streams themselves)."""
+
+    def __init__(self, ptr, n):
+        self.__cuda_array_interface__ = {"shape": (n,), "typestr": "<f8", "data": (ptr, False),
+                                         "version": 3, "strides": None}
+
+
+class TorchProblem:
+    """ParOpt.Problem with callbacks on torch tensors in device memory
+    (pcu_problem_create): subclass and implement
+
+        getVarsAndBounds(x, lb, ub)
+        evalObjCon(x) -> (fail, fobj, con)
+        evalObjConGradient(x, g, A) -> fail          A: list of ncon tensors
+        writeOutput(it, x)                           optional
+        evalHvecProduct(x, z, zw, px, hvec) -> fail  optional; z: ncon host values
+        computeQuasiNewtonUpdateCorrection(x, z, zw, s, y) -> fail   optional
+
+    Every vector is a float64 CUDA tensor viewing the library's own memory: fill the
+    outputs in place (g.copy_(...), A[j].copy_(...)); nothing is copied between host
+    and device.  fobj and con may be Python floats, 0-d tensors or a 1-D tensor; they
+    reach the host in one device->host copy per evalObjCon.  As in Problem, an
+    optional callback is registered only when the subclass defines it.
+
+    The callbacks run with torch's current stream set to the context's stream
+    (Context.stream), after that stream has been made to wait on the stream that was
+    current when the optimizer was called, so tensors filled just before optimize()
+    are complete when a callback reads them.  Multi-rank problems reduce their
+    partial sums with Context.allreduce_sum.
+
+    `x` handed to different callbacks may be different buffers holding the same
+    values (the optimizer exchanges vectors instead of copying them): do not cache
+    results by tensor or pointer.
+
+    An exception in a callback prints its traceback and reports a failed
+    evaluation.  Later callbacks of the same run then fail without calling the
+    subclass, and InteriorPoint / TrustRegion raise RuntimeError from the first
+    exception when the run returns."""
+
+    def __init__(self, ctx, nvars, ncon, ninequality=-1, nwinequality=-1,
+                 use_lower=True, use_upper=True, weighting=None):
+        import torch
+        self.ctx = ctx
+        self.lib = ctx.lib
+        self.nvars, self.ncon = int(nvars), int(ncon)
+        self.device = torch.device("cuda", ctx.device)
+        w = _lib.Weighting()
+        if weighting:
+            for k, v in weighting.items():
+                setattr(w, k, v)
+        self._w = w
+        self._views = {}
+        self._error = None
+        self._ready = None  # event: the caller's stream at the entry of a callback
+        self._empty = torch.empty(0, dtype=torch.float64, device=self.device)
+        cb = _lib.Callbacks()
+        cb.user = None
+        cb.get_vars_and_bounds = _lib.GET_VARS_CB(self._get_vars)
+        cb.eval_obj_con = _lib.EVAL_OBJ_CB(self._eval_obj)
+        cb.eval_obj_con_gradient = _lib.EVAL_GRAD_CB(self._eval_grad)
+        if hasattr(self, "computeQuasiNewtonUpdateCorrection"):
+            cb.qn_update_correction = _lib.QN_CORR_CB(self._qn_correction)
+        if hasattr(self, "writeOutput"):
+            cb.write_output = _lib.WRITE_OUT_CB(self._write_output)
+        if hasattr(self, "evalHvecProduct"):
+            cb.eval_hvec_product = _lib.HVEC_CB(self._eval_hvec)
+        self._cb = cb
+        self.h = self.lib.pcu_problem_create(
+            ctx.h, self.nvars, self.ncon, int(ninequality), int(nwinequality),
+            int(use_lower), int(use_upper), C.byref(self._w), C.byref(self._cb))
+        if not self.h:
+            raise RuntimeError("paropt_b200: problem creation failed")
+
+    def _vec(self, h):
+        """Zero-copy tensor view of a pcu_vec, cached by handle and device pointer: the
+        quasi-Newton memory exchanges buffers, so a handle can change its storage."""
+        if not h:
+            return self._empty
+        ptr = int(self.lib.pcu_vec_device_ptr(h) or 0)
+        key = (h, ptr)
+        t = self._views.get(key)
+        if t is None:
+            import torch
+            n = int(self.lib.pcu_vec_size(h))
+            t = (torch.as_tensor(_DeviceArray(ptr, n), device=self.device)
+                 if n > 0 and ptr else self._empty)
+            self._views[key] = t
+        return t
+
+    def _call(self, fn, *args):
+        """Runs one callback body on the context's stream; 0 / 1 for the library."""
+        if self._error is not None:
+            return 1
+        import torch
+        try:
+            stream = self.ctx.stream
+            cur = torch.cuda.current_stream(self.device)
+            if cur != stream:
+                if self._ready is None:
+                    self._ready = torch.cuda.Event()
+                self._ready.record(cur)
+                stream.wait_event(self._ready)
+            with torch.cuda.stream(stream):
+                return int(fn(*args) or 0)
+        except Exception as e:  # report, do not unwind through C (ParOpt.pyx:528-531)
+            import traceback
+            traceback.print_exc()
+            self._error = e
+            return 1
+
+    def take_callback_error(self):
+        """The exception a callback raised in the last run (None if none), cleared."""
+        e, self._error = self._error, None
+        return e
+
+    def _get_vars(self, user, x, lb, ub):
+        return self._call(lambda: self.getVarsAndBounds(self._vec(x), self._vec(lb),
+                                                        self._vec(ub)))
+
+    def _eval_obj(self, user, x, fobj, cons):
+        def body():
+            fail, f, con = self.evalObjCon(self._vec(x))
+            vals = self._host_values(f, con)
+            fobj[0] = vals[0]
+            for i in range(self.ncon):
+                cons[i] = vals[i + 1]
+            return fail
+        return self._call(body)
+
+    def _host_values(self, f, con):
+        """[fobj, con...] as host floats: tensor entries are gathered into one device
+        buffer and copied to the host once."""
+        import torch
+        out = [None] * (self.ncon + 1)
+        dev = []  # (slot, tensor)
+        if torch.is_tensor(f):
+            dev.append((0, f.reshape(1)))
+        else:
+            out[0] = float(f)
+        if torch.is_tensor(con):
+            if con.numel() != self.ncon:
+                raise ValueError("evalObjCon returned %d constraints, expected %d"
+                                 % (con.numel(), self.ncon))
+            if self.ncon:
+                dev.append((1, con.reshape(-1)))
+        else:
+            con = list(con) if con is not None else []
+            if len(con) != self.ncon:
+                raise ValueError("evalObjCon returned %d constraints, expected %d"
+                                 % (len(con), self.ncon))
+            for i, c in enumerate(con):
+                if torch.is_tensor(c):
+                    dev.append((i + 1, c.reshape(1)))
+                else:
+                    out[i + 1] = float(c)
+        if dev:
+            buf = torch.empty(self.ncon + 1, dtype=torch.float64, device=self.device)
+            for slot, t in dev:
+                buf[slot:slot + t.numel()].copy_(t)
+            host = buf.cpu().tolist()  # the one synchronisation
+            for slot, t in dev:
+                out[slot:slot + t.numel()] = host[slot:slot + t.numel()]
+        return out
+
+    def _eval_grad(self, user, x, g, Ac):
+        return self._call(lambda: self.evalObjConGradient(
+            self._vec(x), self._vec(g), [self._vec(Ac[i]) for i in range(self.ncon)]))
+
+    def _eval_hvec(self, user, x, z, zw, px, hvec):
+        zz = np.array([z[i] for i in range(self.ncon)])
+        return self._call(lambda: self.evalHvecProduct(
+            self._vec(x), zz, self._vec(zw), self._vec(px), self._vec(hvec)))
+
+    def _qn_correction(self, user, x, z, zw, s, y):
+        zz = np.array([z[i] for i in range(self.ncon)])
+        return self._call(lambda: self.computeQuasiNewtonUpdateCorrection(
+            self._vec(x), zz, self._vec(zw), self._vec(s), self._vec(y)))
+
+    def _write_output(self, user, it, x):
+        return self._call(lambda: self.writeOutput(int(it), self._vec(x)))
+
+    def callback_ms(self):
+        """Device milliseconds spent inside the callbacks (events on the context's stream)."""
+        return float(self.lib.pcu_problem_callback_ms(self.h))
+
+    def transfer_bytes(self):
+        a, b = C.c_int64(), C.c_int64()
+        self.lib.pcu_problem_transfer_bytes(self.h, C.byref(a), C.byref(b))
+        return a.value, b.value
+
+    @property
+    def h2d_bytes(self):
+        return self.transfer_bytes()[0]
+
+    @property
+    def d2h_bytes(self):
+        return self.transfer_bytes()[1]
+
+    def free(self):
+        if self.h:
+            self._views.clear()
+            self.lib.pcu_problem_destroy(self.h)
+            self.h = None
+
+
+class AutogradProblem(TorchProblem):
+    """A TorchProblem whose derivatives come from torch.autograd: subclass and
+    implement getVarsAndBounds(x, lb, ub) and objcon(x) -> (f, c) with f a 0-d tensor
+    and c a 1-D tensor (or list) of the ncon constraints, written in differentiable
+    torch operations.  The gradients are one backward pass per output through a
+    retained graph; the Hessian-vector product (use_hvec_product) is the double
+    backward of the Lagrangian L = f - z^T c (the reference's sign convention; the
+    weighting rows are linear and add nothing)."""
+
+    def _outputs(self, x):
+        f, c = self.objcon(x)
+        cs = [c[i] for i in range(self.ncon)]
+        return f, cs
+
+    def evalObjCon(self, x):
+        import torch
+        with torch.no_grad():
+            f, c = self.objcon(x)
+        return 0, f, c
+
+    def evalObjConGradient(self, x, g, A):
+        import torch
+        with torch.enable_grad():
+            xr = x.detach().requires_grad_(True)
+            f, cs = self._outputs(xr)
+            outs = [f] + cs
+            for k, (out, dst) in enumerate(zip(outs, [g] + list(A))):
+                grad = None
+                if torch.is_tensor(out) and out.requires_grad:
+                    (grad,) = torch.autograd.grad(out, xr, retain_graph=k + 1 < len(outs),
+                                                  allow_unused=True)
+                if grad is None:
+                    dst.zero_()
+                else:
+                    dst.copy_(grad)
+        return 0
+
+    def evalHvecProduct(self, x, z, zw, px, hvec):
+        import torch
+        with torch.enable_grad():
+            xr = x.detach().requires_grad_(True)
+            f, cs = self._outputs(xr)
+            L = f
+            for zj, cj in zip(z, cs):
+                L = L - float(zj) * cj
+            hv = None
+            if torch.is_tensor(L) and L.requires_grad:
+                (gL,) = torch.autograd.grad(L, xr, create_graph=True)
+                if gL.requires_grad:
+                    (hv,) = torch.autograd.grad(gL, xr, grad_outputs=px, allow_unused=True)
+            if hv is None:
+                hvec.zero_()
+            else:
+                hvec.copy_(hv)
+        return 0
+
+
+def _raise_callback_error(prob, rc, what):
+    """RuntimeError for a failed library call, chained to the exception a
+    TorchProblem callback raised during it (the library may absorb a failed
+    evaluation, e.g. by shortening a line-search step)."""
+    take = getattr(prob, "take_callback_error", None)
+    err = take() if take is not None else None
+    if err is not None:
+        raise RuntimeError("paropt_b200: %s: a problem callback raised %s: %s"
+                           % (what, type(err).__name__, err)) from err
+    _check(rc, what)
+
+
 class BuiltinProblem:
     """Synthetic problems shipped with the library: GPU-resident
     (pcu_problem_create_sepquad / _rosenbrock) or, with host=True, the same
@@ -638,14 +938,15 @@ class InteriorPoint:
         _check(self.lib.pcu_ip_reset_quasi_newton(self.h), "resetQuasiNewtonHessian")
 
     def optimize(self):
-        _check(self.lib.pcu_ip_optimize(self.h), "optimize")
+        _raise_callback_error(self.prob, self.lib.pcu_ip_optimize(self.h), "optimize")
 
     def begin(self):
-        _check(self.lib.pcu_ip_begin(self.h), "begin")
+        _raise_callback_error(self.prob, self.lib.pcu_ip_begin(self.h), "begin")
 
     def iterate(self, n=1):
         conv = C.c_int()
-        _check(self.lib.pcu_ip_iterate(self.h, int(n), C.byref(conv)), "iterate")
+        _raise_callback_error(self.prob, self.lib.pcu_ip_iterate(self.h, int(n), C.byref(conv)),
+                              "iterate")
         return bool(conv.value)
 
     def status(self):
@@ -767,7 +1068,8 @@ class TrustRegion:
             raise ValueError("option %s=%r is not available" % (name, value))
 
     def optimize(self):
-        _check(self.lib.pcu_tr_optimize(self.h), "trust-region optimize")
+        _raise_callback_error(self.prob, self.lib.pcu_tr_optimize(self.h),
+                              "trust-region optimize")
 
     def converged(self):
         return int(self.lib.pcu_tr_status(self.h)) == 1
