@@ -458,6 +458,11 @@ int pcu_ip_setup_kkt_diag(pcu_ip *ip, int use_qn);               /* IP.cpp:1832 
 int pcu_ip_setup_kkt(pcu_ip *ip, int use_qn);                    /* IP.cpp:2634 */
 int pcu_ip_kkt_step(pcu_ip *ip, int res, int step, int use_qn);  /* IP.cpp:2700 */
 int pcu_ip_add_kkt_res_step(pcu_ip *ip, int step, int res);      /* IP.cpp:1451 */
+/* The KKT solve of the default iteration (one refinement step, done in the column
+   space of [A|Z]) at the current point and barrier, right-hand side from the
+   variables, dense algebra on the device (on_device = 1) or on the host; needs
+   1 <= ncon + quasi-Newton width <= 32.  res receives the dense residual only. */
+int pcu_ip_kkt_solve(pcu_ip *ip, int res, int step, int on_device); /* IP.cpp:4971 */
 int pcu_ip_max_step(pcu_ip *ip, double tau, int step, double *max_x,
                     double *max_z);                              /* IP.cpp:2942 */
 int pcu_ip_comp_step(pcu_ip *ip, double alpha_x, double alpha_z, int step,

@@ -221,6 +221,7 @@ SIGNATURES = {
     "pcu_ip_setup_kkt": (C.c_int, [VP, C.c_int]),
     "pcu_ip_kkt_step": (C.c_int, [VP, C.c_int, C.c_int, C.c_int]),
     "pcu_ip_add_kkt_res_step": (C.c_int, [VP, C.c_int, C.c_int]),
+    "pcu_ip_kkt_solve": (C.c_int, [VP, C.c_int, C.c_int, C.c_int]),
     "pcu_ip_max_step": (C.c_int, [VP, C.c_double, C.c_int, c_double_p, c_double_p]),
     "pcu_ip_comp_step": (C.c_int, [VP, C.c_double, C.c_double, C.c_int, c_double_p]),
     "pcu_ip_merit_init_deriv": (C.c_int, [VP, C.c_double, c_double_p, c_double_p]),

@@ -573,6 +573,23 @@ int pcu_ip_add_kkt_res_step(pcu_ip *ip, int step, int res) {
                            dots.data() + ip->ncon);
 }
 
+int pcu_ip_kkt_solve(pcu_ip *ip, int res, int step, int on_device) {
+  Vars *r = bundle(ip, res), *s = bundle(ip, step);
+  if (!r || !s) return 1;
+  if (ip->ensure_qn()) return 1;
+  if (on_device && !ip->ctx->chain_ok()) return 1;
+  ip->refresh_penalties();
+  const int m = ip->ncon + (ip->qn ? ip->qn->size() : 0);
+  if (m < 1 || m > PCU_DENSE_MAXM) return 1;
+  std::vector<double> vtp(m + 1);
+  double tau = ip->opt.min_fraction_to_boundary;
+  if (1.0 - ip->barrier_param >= tau) tau = 1.0 - ip->barrier_param;
+  const int rc = ip->kktChain(ip->variables, *r, *s, 1, ip->barrier_param, tau, vtp.data(),
+                              on_device);
+  ip->stats_ready = 0;
+  return rc;
+}
+
 int pcu_ip_max_step(pcu_ip *ip, double tau, int step, double *max_x,
                     double *max_z) {
   Vars *s = bundle(ip, step);

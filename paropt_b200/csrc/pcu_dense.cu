@@ -1,8 +1,8 @@
 // pcu_dense.cu -- device side of pcu_dense.cuh: a single-CTA kernel that runs the
-// small dense algebra of the KKT solve between two streaming passes, so that the
-// iteration's chain  Gram -> pass 2 + residual -> pass 2 + statistics  needs no host
-// round trip (LU of G and Ce, SMW coefficient assembly, dense residuals, fed by the
-// in-stream all-reduce / all-gather result).
+// small dense algebra of the default iteration's KKT solve between the Gram pass and
+// the one pass that applies the step, so that the chain  DiagRhsF -> Gram -> dense ->
+// Pass2SVF  needs no host round trip (LU of G and Ce, SMW coefficients, dense
+// residuals, the refinement in the column space of [A|Z]).
 //
 // The flat work buffer (<= 5k doubles) is staged in shared memory by all threads, warp
 // 0 runs the lane-parallel algorithm of pcu_dense.cuh on it (matrices of at most
@@ -16,36 +16,28 @@
 #define PCU_DENSE_THREADS 128
 
 __global__ void __launch_bounds__(PCU_DENSE_THREADS, 1)
-    pcu_dense_kernel(double *buf, const DenseOff o, const int phase, const double *Sin,
-                     const double *red, const int world, const int stride, long long *tick) {
+    pcu_dense_kernel(double *buf, const DenseOff o, const double *Sin, long long *tick) {
   extern __shared__ double2 dense_smem2[];
   double *w = reinterpret_cast<double *>(dense_smem2);
   double *scratch = w + o.total;
   const int tid = threadIdx.x;
   if (tick && tid == 0) tick[0] = clock64();
-  // phase 0 needs the inputs only (the rest is produced here); phase 1 everything
-  const int n_in = phase == 0 ? o.S : o.total;
-  for (int i = tid; i < n_in; i += PCU_DENSE_THREADS) w[i] = buf[i];
-  if (phase == 0) {
-    const int nS = o.ld * o.ld;
-    for (int i = tid; i < nS; i += PCU_DENSE_THREADS) w[o.S + i] = Sin[i];
-  }
+  // the inputs only (the rest is produced here)
+  for (int i = tid; i < o.S; i += PCU_DENSE_THREADS) w[i] = buf[i];
+  const int nS = o.ld * o.ld;
+  for (int i = tid; i < nS; i += PCU_DENSE_THREADS) w[o.S + i] = Sin[i];
   __syncthreads();
   if (tick && tid == 0) tick[1] = clock64();
-  if (tid < 32) {
-    if (phase == 0) pcu_dense_phase_a(w, o, scratch, tick);
-    else pcu_dense_phase_b(w, o, red, world, stride, scratch);
-  }
+  if (tid < 32) pcu_dense_solve(w, o, scratch, tick);
   __syncthreads();
   if (tick && tid == 0) tick[4] = clock64();
   for (int i = o.S + tid; i < o.total; i += PCU_DENSE_THREADS) buf[i] = w[i];
   if (tick && tid == 0) tick[5] = clock64();
 }
 
-// Enqueues one phase on `stream`.  buf: device work buffer (layout `o`); Sin: Gram
-// result (phase 0); red / world / stride: rank-ordered partial reductions (phase 1).
-int pcu_dense_enqueue(cudaStream_t stream, double *buf, const DenseOff &o, int phase,
-                      const double *Sin, const double *red, int world, int stride) {
+// Enqueues pcu_dense_solve on `stream`.  buf: device work buffer (layout `o`, inputs
+// in place); Sin: Gram result.
+int pcu_dense_enqueue(cudaStream_t stream, double *buf, const DenseOff &o, const double *Sin) {
   const size_t smem = sizeof(double) * (size_t)(o.total + PCU_DENSE_SCRATCH(o.c, o.q));
   if (smem > 48 * 1024) {
     static bool raised[64] = {false};
@@ -62,30 +54,23 @@ int pcu_dense_enqueue(cudaStream_t stream, double *buf, const DenseOff &o, int p
   static long long *ticks = nullptr;
   static int tick_calls = 0;
   const bool profile = getenv("PCU_DENSE_TICKS") != nullptr;
-  if (profile && !ticks) cudaMalloc(&ticks, 16 * sizeof(long long));
-  pcu_dense_kernel<<<1, PCU_DENSE_THREADS, smem, stream>>>(buf, o, phase, Sin, red, world, stride,
-                                                           profile ? ticks + 8 * phase : nullptr);
-  if (profile && ++tick_calls % 40 < 2) {
+  if (profile && !ticks) cudaMalloc(&ticks, 8 * sizeof(long long));
+  pcu_dense_kernel<<<1, PCU_DENSE_THREADS, smem, stream>>>(buf, o, Sin,
+                                                           profile ? ticks : nullptr);
+  if (profile && ++tick_calls % 20 < 1) {
     cudaStreamSynchronize(stream);
-    long long host_ticks[16];
-    cudaMemcpy(host_ticks, ticks, sizeof(host_ticks), cudaMemcpyDeviceToHost);
-    const long long *t = host_ticks + 8 * phase;
-    fprintf(stderr, "dense phase %d (c=%d q=%d) cycles: stage-in %lld, setup %lld, step %lld, rest %lld, "
-            "stage-out %lld, total %lld\n", phase, o.c, o.q, t[1] - t[0], phase == 0 ? t[2] - t[1] : 0,
-            phase == 0 ? t[3] - t[2] : 0, phase == 0 ? t[4] - t[3] : t[4] - t[1], t[5] - t[4],
-            t[5] - t[0]);
+    long long t[8];
+    cudaMemcpy(t, ticks, sizeof(t), cudaMemcpyDeviceToHost);
+    fprintf(stderr, "dense kernel (c=%d q=%d) cycles: stage-in %lld, setup %lld, step %lld, "
+            "refinement %lld, stage-out %lld, total %lld\n", o.c, o.q, t[1] - t[0], t[2] - t[1],
+            t[3] - t[2], t[4] - t[3], t[5] - t[4], t[5] - t[0]);
   }
   return cudaGetLastError() == cudaSuccess ? 0 : 1;
 }
 
-// The same two phases on the host (checker of the device path).
-void pcu_dense_host(double *w, const DenseOff &o, int phase, const double *Sin,
-                    const double *red, int world, int stride) {
+// The same solve on the host (the KKT solve's host route: PCU_NO_CHAIN, several GPUs).
+void pcu_dense_host(double *w, const DenseOff &o, const double *Sin) {
   double scratch[PCU_DENSE_SCRATCH(PCU_DENSE_MAXM / 2, PCU_DENSE_MAXM / 2) + 8 * PCU_DENSE_MAXM];
-  if (phase == 0) {
-    for (int i = 0; i < o.ld * o.ld; i++) w[o.S + i] = Sin[i];
-    pcu_dense_phase_a(w, o, scratch);
-  } else {
-    pcu_dense_phase_b(w, o, red, world, stride, scratch);
-  }
+  for (int i = 0; i < o.ld * o.ld; i++) w[o.S + i] = Sin[i];
+  pcu_dense_solve(w, o, scratch);
 }

@@ -1,18 +1,20 @@
 // pcu_dense.cuh -- the small dense algebra of the KKT solve (the c x c matrix G,
 // the q x q matrix Ce, the Sherman-Morrison-Woodbury coefficients) as ONE piece of
-// host/device code, so that the chain
-//     Gram pass -> [this] -> pass 2 + refinement residual -> [this] -> pass 2 + statistics
-// runs on the device without a host round trip (pcu_dense.cu: single-CTA kernel on
-// a flat work buffer staged in shared memory), while every other configuration keeps
-// the host path of pcu_ip_solve.cu.  Reference: setUpKKTDiagSystem's G (IP.cpp:1932-
-// 1969, dgetrf), setUpKKTSystem's Ce (IP.cpp:2646-2664, dgetrf), the dense part of
-// solveKKTDiagSystem (IP.cpp:2150-2170, 2288-2306) and of computeKKTStep
+// host/device code, so that the default iteration's solve
+//     Gram pass -> [pcu_dense_solve] -> Pass2SVF (the step + its statistics)
+// runs either on the device without a host round trip (pcu_dense.cu: single-CTA kernel
+// on a flat work buffer staged in shared memory) or, with the same statements, on the
+// host (pcu_dense_host).  The one iterative-refinement step of that solve is done here,
+// in the column space of V = [A|Z] (pcu_dense_solve).  Reference: setUpKKTDiagSystem's
+// G (IP.cpp:1932-1969, dgetrf), setUpKKTSystem's Ce (IP.cpp:2646-2664, dgetrf), the
+// dense part of solveKKTDiagSystem (IP.cpp:2150-2170, 2288-2306) and of computeKKTStep
 // (IP.cpp:2716-2735), computeKKTRes / addKKTResStep's dense residual
-// (IP.cpp:1401-1407, 1535-1541), ParOptLBFGS::mult's compact solve (QN.cpp:398-412).
+// (IP.cpp:1401-1407, 1535-1541), ParOptLBFGS::mult's compact solve (QN.cpp:398-412),
+// the refinement loop (IP.cpp:4985-4991).
 //
-// Same statements as the host path; the device replaces the divisions on its critical
-// path by reciprocals (<= 1 ulp each), so chain and host path agree to round-off
-// (tests/test_gpu_gram_paths.py holds the two histories to 1e-12).
+// The device replaces the divisions on its critical path by reciprocals (<= 1 ulp
+// each), so the device and host runs agree to round-off (tests/test_gpu_gram_paths.py
+// holds the two histories to 1e-12).
 #pragma once
 
 #include <cuda_runtime.h>
@@ -38,7 +40,8 @@ struct DenseOff {
   int bz, bs, bt, bzs, bzt;                  // dense residual (right-hand side)
   int yz, ys, yt, yzs, yzt;                  // dense step (accumulated)
   int r, vtp;                                // [A|Z]^T t1 of the current solve; [A|Z]^T step
-  int coefA, coefB;                          // alpha | beta of pass 2 + residual; alpha of the last pass
+  int coef, alpha2;                          // alpha of the first solve, then of the whole step
+                                             // (the pass's table); alpha of the refinement
   int total;
 };
 
@@ -67,8 +70,8 @@ static inline DenseOff pcu_dense_offsets(int c, int q, int ld) {
   o.yz = take(c); o.ys = take(c); o.yt = take(c); o.yzs = take(c); o.yzt = take(c);
   o.r = take(o.m); o.vtp = take(o.m);
   p = (p + 1) & ~1;
-  o.coefA = take(2 * PCU_DENSE_MAXM);
-  o.coefB = take(PCU_DENSE_MAXM);
+  o.coef = take(PCU_DENSE_MAXM);
+  o.alpha2 = take(PCU_DENSE_MAXM);
   o.total = (p + 1) & ~1;
   return o;
 }
@@ -421,47 +424,59 @@ PCU_HDN void pcu_dense_step(double *w, const DenseOff &o, int accumulate, double
   PCU_SYNC();
 }
 
-// Phase A: everything between the Gram pass and the pass that applies the first
-// solve and emits the refinement residual.  w[S] holds the Gram result (ld x ld, lower
-// triangle, row m = [A|Z]^T t1 of the first solve).  scratch: >= max(c q, 2 m + 5 c).
-PCU_HD void pcu_dense_phase_a(double *w, const DenseOff &o, double *scratch,
-                              long long *tick = nullptr) {
+// The KKT solve of the default iteration (one refinement step) between the Gram pass and
+// the one pass that applies it.  w[S] holds the Gram result (ld x ld, lower triangle,
+// row m = [A|Z]^T t1 of the first solve, t1 = D0^-1 d1).  scratch: >= max(c q, 2 m + 5 c).
+//
+// The first solve is p1 = D0^-1 (d1 + V alpha1), V = [A|Z].  The x row of its
+// residual r - K p1 is (Pass2R1F's rx with lin = V beta, beta = (z + pz, kap))
+//     t = A (pz - alpha1_A) + Z (kap - alpha1_Z) = V delta,
+//     delta_A = 0 exactly (alpha1_A is pz),  delta_Z = kap - alpha1_Z,
+// and the bound and weighting rows of that residual vanish given px.  So the
+// refinement solve's reductions are r' = V^T D0^-1 t = S delta, its dense rows are the
+// dense residual at p1, and the refined step is
+//     p = p1 + D0^-1 (t + V alpha2) = D0^-1 (d1 + V (alpha1 + delta + alpha2)):
+// one pass with the table (alpha1_A + alpha2_A, kap + alpha2_Z) left in w[coef].  What
+// this drops against refining the N-sized residual elementwise is the rounding of the
+// elementwise operations (relative eps per element); the correction the refinement is
+// for -- the error of the solves with G and Ce -- lives in this column space and is kept.
+PCU_HD void pcu_dense_solve(double *w, const DenseOff &o, double *scratch,
+                            long long *tick = nullptr) {
   const int c = o.c, q = o.q, ld = o.ld, m = o.m;
   PCU_PFOR(j, 0, m) w[o.r + j] = w[o.S + m + ld * j];
   PCU_SYNC();
   pcu_dense_setup(w, o, scratch);
   PCU_TICK(tick, 2);
   pcu_dense_residual(w, o, 0);
-  double *alpha = w + o.coefA, *beta = alpha + PCU_DENSE_MAXM;
+  double *alpha = w + o.coef, *alpha2 = w + o.alpha2;
   pcu_dense_step(w, o, 0, alpha, scratch);
   PCU_TICK(tick, 3);
-  // coefficients of the linearised residual: z + pz for A, the compact
-  // quasi-Newton solve kap = d0 M^-1 d0 (Z^T p) for Z (IP.cpp:1474-1476)
-  PCU_PFOR(j, 0, c) beta[j] = w[o.vz + j] + w[o.yz + j];
+  // kap = d0 M^-1 d0 (Z^T p1), the compact quasi-Newton solve (IP.cpp:1474-1476):
+  // alpha_Z takes kap, alpha2_Z holds delta_Z until the refinement step overwrites it
   if (q > 0) {
-    double *kap = scratch;
+    double *kap = alpha2 + c;
     PCU_PFOR(i, 0, q) {
       kap[i] = w[o.vtp + c + i] * w[o.d0 + i];
       w[o.minv + i] = pcu_dense_rcp(w[o.Mf + i * (q + 1)]);
     }
     PCU_SYNC();
     pcu_dense_lu_solve(q, w + o.Mf, w + o.mpiv, w + o.minv, kap);
-    PCU_PFOR(i, 0, q) beta[c + i] = kap[i] * w[o.d0 + i];
+    PCU_PFOR(i, 0, q) {
+      const double kz = kap[i] * w[o.d0 + i];
+      kap[i] = kz - alpha[c + i];
+      alpha[c + i] = kz;
+    }
   }
   PCU_SYNC();
-  pcu_dense_residual(w, o, 1);  // right-hand side of the refinement solve
-}
-
-// Phase B: between that pass (whose reductions r' = [A|Z]^T t1' arrive as `world`
-// rank-ordered partial vectors of `stride` doubles) and the last pass.
-PCU_HD void pcu_dense_phase_b(double *w, const DenseOff &o, const double *red, int world,
-                              int stride, double *scratch) {
-  PCU_PFOR(i, 0, o.m) {
-    double v = red[i];
+  pcu_dense_residual(w, o, 1);  // dense rows of the refinement's right-hand side
+  PCU_PFOR(i, 0, m) {           // r' = S delta
+    double v = 0.0;
 #pragma unroll 1
-    for (int rk = 1; rk < world; rk++) v += red[(size_t)rk * stride + i];
+    for (int j = 0; j < q; j++) v += w[o.S + i + ld * (c + j)] * alpha2[c + j];
     w[o.r + i] = v;
   }
   PCU_SYNC();
-  pcu_dense_step(w, o, 1, w + o.coefB, scratch);
+  pcu_dense_step(w, o, 1, alpha2, scratch);
+  PCU_PFOR(j, 0, m) alpha[j] += alpha2[j];
+  PCU_SYNC();
 }

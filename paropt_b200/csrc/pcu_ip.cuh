@@ -182,11 +182,11 @@ struct pcu_ip {
   int force_direct_dots = 0;  // debugging: recompute [A|Z]^T p with multi-dots
   int opt_no_rhsgram = 0;     // debugging: keep the first solve's pass 1 out of the Gram pass
   int opt_no_fuse2s = 0;      // debugging: keep the step statistics in their own pass
-  int stats_ready = 0;        // Pass2SF left the step statistics in stats_out
+  int stats_ready = 0;        // Pass2SF / Pass2SVF left the step statistics in stats_out
   double stats_tau_used = 0.0;
   double stats_out[32];
   int opt_no_wide = 0;        // debugging: more than 32 columns stay on the register-fed pass 2
-  int opt_no_fuse21 = 0;      // debugging: keep pass 2 and the next pass 1 separate
+  int opt_no_fuse21 = 0;      // debugging: refine elementwise, pass 2 and the next pass 1 separate
   // residual statistics of the NEXT iteration taken by the update passes (ResF layout)
   double upd_sums[11], upd_max[5], upd_min[2];
   int upd_stats_valid = 0;
@@ -259,7 +259,8 @@ struct pcu_ip {
   int setUpKKTDiagSystem(Vars &vars, int use_qn, int identity);
   int setUpKKTDiagRhs(Vars &vars, int use_qn, double mu);
   int setUpKKTSystem(Vars &vars, int use_qn, const double *gdiag, int with_rhs = 0);
-  int kktChain(Vars &vars, Vars &b, Vars &y, int use_qn, double mu, double tau, double *VTp);
+  int kktChain(Vars &vars, Vars &b, Vars &y, int use_qn, double mu, double tau, double *VTp,
+               int on_device);
   int computeKKTStep(Vars &vars, Vars &res, Vars &step, int use_qn,
                      int accumulate, double *VTp, int emit_res, double mu_res,
                      int *emitted, int rhs_from_vars = 0, double stats_tau = -1.0);

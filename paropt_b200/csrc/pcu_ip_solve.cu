@@ -498,36 +498,40 @@ int pcu_ip::computeKKTStep(Vars &vars, Vars &b, Vars &y, int use_qn,
 
 // ------------------------------------------------------------------ kktChain
 // The KKT solve of a default iteration (monotone barrier, one refinement step,
-// ncon + q <= 32) as ONE stream-ordered chain without a host round trip:
-//   DiagRhsF -> Gram (+ in-stream all-reduce) -> dense phase A -> Pass2R1F
-//   (+ in-stream all-gather of its partials) -> dense phase B -> Pass2SF -> fetch.
-// The small dense algebra (LU of G and Ce, SMW coefficients, dense residuals) runs in
-// pcu_dense_kernel on a flat device buffer; the two passes read their coefficient
-// tables from it.  Same arithmetic as setUpKKTDiagRhs + setUpKKTSystem +
-// computeKKTStep x 2 (IP.cpp:1832-1971, 2634-2737, 4971-4991), which remain the path of
-// every other configuration (and of PCU_NO_CHAIN).
-int pcu_dense_enqueue(cudaStream_t stream, double *buf, const DenseOff &o, int phase,
-                      const double *Sin, const double *red, int world, int stride);
+// ncon + q <= 32, right-hand side from the variables) as ONE stream-ordered chain:
+//   DiagRhsF -> Gram (+ all-reduce) -> pcu_dense_solve -> Pass2SVF -> fetch.
+// The iterative refinement is done in the column space of [A|Z] by the small dense
+// algebra (pcu_dense.cuh: pcu_dense_solve), so one pass applies the refined step and
+// takes its statistics.  on_device: the dense algebra runs in pcu_dense_kernel on a
+// flat device buffer, the pass reads its coefficients from the constant bank, and the
+// chain needs no host round trip; otherwise the same statements run on the host
+// between the Gram result and the pass.  Same arithmetic as setUpKKTDiagRhs +
+// setUpKKTSystem + computeKKTStep x 2 (IP.cpp:1832-1971, 2634-2737, 4971-4991) up to
+// the rounding of the refinement residual's elementwise operations.
+int pcu_dense_enqueue(cudaStream_t stream, double *buf, const DenseOff &o, const double *Sin);
+void pcu_dense_host(double *w, const DenseOff &o, const double *Sin);
 
 int pcu_ip::kktChain(Vars &vars, Vars &b, Vars &y, int use_qn, double mu, double tau,
-                     double *VTp) {
+                     double *VTp, int on_device) {
   const int q = (qn && use_qn) ? qn->size() : 0;
   const int m = ncon + q;
+  if (m < 1 || m > PCU_DENSE_MAXM) return 1;
   sq = q;
   stats_ready = 0;
   pass1_ready = 0;
   if (setUpKKTDiagRhs(vars, use_qn, mu)) return 1;
-  // ---- inputs of the dense kernel (host -> device, stream-ordered, 1-7 KB)
+  // ---- inputs of the dense algebra (1-7 KB)
   const int ld = 8 * ((m + 1 + 7) / 8);
   const DenseOff o = pcu_dense_offsets(ncon, q, ld);
-  if (!dense_dev || dense_cap < o.total) {
+  if (!dense_host || dense_cap < o.total) {
     if (dense_dev) cudaFree(dense_dev);
     if (dense_host) cudaFreeHost(dense_host);
+    dense_dev = nullptr;
     dense_cap = pcu_dense_offsets(ncon, qn ? qn->max_size() : 0, 40).total + 64;
     if (dense_cap < o.total) dense_cap = o.total + 64;
-    PCU_CUDA_OK(cudaMalloc(&dense_dev, sizeof(double) * dense_cap));
     PCU_CUDA_OK(cudaMallocHost(&dense_host, sizeof(double) * dense_cap));
   }
+  if (on_device && !dense_dev) PCU_CUDA_OK(cudaMalloc(&dense_dev, sizeof(double) * dense_cap));
   double *h = dense_host;
   h[o.mu] = mu;
   h[o.mu + 1] = 0.0;
@@ -547,8 +551,9 @@ int pcu_ip::kktChain(Vars &vars, Vars &b, Vars &y, int use_qn, double mu, double
     memcpy(h + o.Mf, qn->Mf.data(), sizeof(double) * q * q);
     for (int i = 0; i < q; i++) h[o.mpiv + i] = (double)qn->piv[i];
   }
-  PCU_CUDA_OK(cudaMemcpyAsync(dense_dev, h, sizeof(double) * o.S, cudaMemcpyHostToDevice,
-                              ctx->stream));
+  if (on_device)
+    PCU_CUDA_OK(cudaMemcpyAsync(dense_dev, h, sizeof(double) * o.S, cudaMemcpyHostToDevice,
+                                ctx->stream));
   // ---- Gram pass with the first solve's right-hand side as column m
   ColTable V;
   for (int j = 0; j < ncon; j++) V.p[j] = Ac[j]->d;
@@ -558,93 +563,53 @@ int pcu_ip::kktChain(Vars &vars, Vars &b, Vars &y, int use_qn, double mu, double
   int ldg = 0;
   if (pcu_gram_enqueue(ctx, Vg, m + 1, Dinv->d, Cw->d, wd, nvars, &ldg, d2->d, m)) return 1;
   if (ldg != ld) return 1;
-  if (ctx->world > 1) {
-    NcclApi &api = nccl_api();
-    if (api.AllReduce(ctx->d_big, ctx->d_big, (size_t)ld * ld, ncclFloat64, ncclSum, ctx->comm,
-                      ctx->stream) != ncclSuccess)
-      return 1;
+  // ---- the dense algebra, refinement included
+  if (on_device) {
+    if (ctx->world > 1) {
+      NcclApi &api = nccl_api();
+      if (api.AllReduce(ctx->d_big, ctx->d_big, (size_t)ld * ld, ncclFloat64, ncclSum,
+                        ctx->comm, ctx->stream) != ncclSuccess)
+        return 1;
+    }
+    ctx->prof_begin("dense_kernel");
+    if (pcu_dense_enqueue(ctx->stream, dense_dev, o, ctx->d_big)) return 1;
+    ctx->prof_end();
+    ctx->launches++;
+    // the pass's coefficients: device buffer -> constant bank, stream-ordered
+    PCU_CUDA_OK(cudaMemcpyToSymbolAsync(pcu_chain_coef, dense_dev + o.coef,
+                                        sizeof(double) * PCU_DENSE_MAXM, 0,
+                                        cudaMemcpyDeviceToDevice, ctx->stream));
+    // what the dense kernel produced (dense step, [A|Z]^T p, the factors) goes to the
+    // host BEFORE the pass is enqueued: its reduction flag then implies the copy (the
+    // fetch below polls that flag, it does not synchronise the stream)
+    PCU_CUDA_OK(cudaMemcpyAsync(h + o.S, dense_dev + o.S, sizeof(double) * (o.total - o.S),
+                                cudaMemcpyDeviceToHost, ctx->stream));
+  } else {
+    std::vector<double> Sg((size_t)ld * ld);
+    if (ctx->big_fetch((size_t)ld * ld, Sg.data())) return 1;
+    pcu_dense_host(h, o, Sg.data());
   }
-  ctx->prof_begin("dense_kernel");
-  if (pcu_dense_enqueue(ctx->stream, dense_dev, o, 0, ctx->d_big, nullptr, 1, 0)) return 1;
-  ctx->prof_end();
-  ctx->launches++;
-  // alpha | beta of the next pass: device buffer -> constant bank, stream-ordered
-  PCU_CUDA_OK(cudaMemcpyToSymbolAsync(pcu_chain_coef, dense_dev + o.coefA,
-                                      sizeof(double) * 2 * PCU_DENSE_MAXM, 0,
-                                      cudaMemcpyDeviceToDevice, ctx->stream));
-  // ---- pass 2 of the first solve + refinement residual + pass 1 of the refinement
-  const IPConst k = kconst();
-  double *red1 = nullptr;
-  int mr = 0;
-  auto fused21 = [&](auto ff) -> int {
-    ff.v = vars.dv(); ff.b = b.dv(); ff.y = y.dv();
-    ff.lb = lb->d; ff.ub = ub->d; ff.Dinv = Dinv->d; ff.Cw = Cw->d;
-    ff.d1 = d1->d; ff.g = g->d;
-    ff.d2 = d2->d;
-    ff.d1out = t1->d;
-    ff.V = V;
-    ff.cbank = 0;
-    ff.ncols = m; ff.accumulate = 0; ff.from_vars = 1;
-    ff.b0sig = opt.qn_sigma + ((qn && !opt.sequential_linear_method) ? qn->b0 : 0.0);
-    ff.mu = mu; ff.mu_rhs = mu; ff.k = k;
-    ff.apz = apz_target(0, true);
-    ff.nca = ncon;
-    RedBuf rb = ctx->redbuf(decltype(ff)::NS, 0, 0);
-    red1 = rb.result;
-    mr = decltype(ff)::NS;
-    if (launch_tile(ctx, ff, nvars, wd, rb)) return 1;
-    apz_done(0, ff.apz);
-    return 0;
-  };
-  int rc;
-  if (m <= 8) rc = fused21(Pass2R1F<8>());
-  else if (m <= 16) rc = fused21(Pass2R1F<16>());
-  else if (m <= 24) rc = fused21(Pass2R1F<24>());
-  else rc = fused21(Pass2R1F<32>());
-  if (rc) return 1;
-  std::swap(d1, t1);  // the last pass reads d1' where the fused pass wrote it
-  PCU_CUDA_OK(cudaEventRecord(evs[ev_cur].k1, ctx->stream));
-  const double *red = red1;
-  if (ctx->world > 1) {
-    NcclApi &api = nccl_api();
-    if (api.AllGather(red1, ctx->d_gather, (size_t)mr, ncclFloat64, ctx->comm, ctx->stream) !=
-        ncclSuccess)
-      return 1;
-    red = ctx->d_gather;
-  }
-  ctx->prof_begin("dense_kernel");
-  if (pcu_dense_enqueue(ctx->stream, dense_dev, o, 1, nullptr, red, ctx->world, mr)) return 1;
-  ctx->prof_end();
-  ctx->launches++;
-  PCU_CUDA_OK(cudaMemcpyToSymbolAsync(pcu_chain_coef, dense_dev + o.coefB,
-                                      sizeof(double) * PCU_DENSE_MAXM,
-                                      sizeof(double) * 2 * PCU_DENSE_MAXM,
-                                      cudaMemcpyDeviceToDevice, ctx->stream));
-  // what the dense kernel produced (dense step, [A|Z]^T p, the factors) goes to the
-  // host BEFORE the last pass is enqueued: its reduction flag then implies the copy
-  // (the fetch below polls that flag, it does not synchronise the stream)
-  PCU_CUDA_OK(cudaMemcpyAsync(h + o.S, dense_dev + o.S, sizeof(double) * (o.total - o.S),
-                              cudaMemcpyDeviceToHost, ctx->stream));
-  // ---- pass 2 of the refinement solve, accumulated, + the step statistics
-  Pass2SF fs;
+  // ---- the one pass: the refined step + the step statistics
+  Pass2SVF fs;
   fs.v = vars.dv(); fs.b = b.dv(); fs.y = y.dv();
   fs.lb = lb->d; fs.ub = ub->d; fs.Dinv = Dinv->d; fs.Cw = Cw->d;
   fs.d1 = d1->d; fs.d2 = d2->d; fs.g = g->d;
   fs.V = V;
-  fs.cbank = 2 * PCU_DENSE_MAXM;
+  fs.cbank = on_device ? 0 : -1;
+  if (!on_device)
+    for (int j = 0; j < m; j++) fs.alpha.v[j] = h[o.coef + j];
   fs.ncols = m;
-  fs.accumulate = 1; fs.tau = tau; fs.k = k;
-  fs.apz = apz_target(1, true);
+  fs.accumulate = 0; fs.tau = tau; fs.mu_rhs = mu; fs.k = kconst();
+  fs.apz = apz_target(0, true);
   fs.nca = ncon;
-  RedBuf rb2 = ctx->redbuf(Pass2SF::NS, Pass2SF::NX, Pass2SF::NM);
-  if (launch_tile(ctx, fs, nvars, wd, rb2)) return 1;
-  apz_done(1, fs.apz);
-  double out[PCU_DENSE_MAXM + Pass2SF::NS + Pass2SF::NX + Pass2SF::NM];
-  if (ctx->fetch(out)) return 1;
-  memcpy(stats_out, out + mr, sizeof(double) * (Pass2SF::NS + Pass2SF::NX + Pass2SF::NM));
+  RedBuf rb = ctx->redbuf(Pass2SVF::NS, Pass2SVF::NX, Pass2SVF::NM);
+  if (launch_tile(ctx, fs, nvars, wd, rb)) return 1;
+  apz_done(0, fs.apz);
+  PCU_CUDA_OK(cudaEventRecord(evs[ev_cur].k1, ctx->stream));
+  if (ctx->fetch(stats_out)) return 1;
   stats_ready = 1;
   stats_tau_used = tau;
-  // ---- host mirrors of what the dense kernel produced
+  // ---- host mirrors of what the dense algebra produced
   for (int i = 0; i < ncon; i++) {
     y.z[i] = h[o.yz + i];
     y.s[i] = h[o.ys + i];
@@ -1503,17 +1468,20 @@ int pcu_ip::iterate_once(int *converged) {
   // the solves
   double tau_pre = opt.min_fraction_to_boundary;
   if (1.0 - barrier_param >= tau_pre) tau_pre = 1.0 - barrier_param;
-  // The device chain is the default on one GPU (same speed as the host path: 51 + 17 us
-  // of dense kernel against two flag-polled host round trips); across GPUs the host
-  // path is faster (measured at 8 GPUs: 1.94 against 2.04 ms per iteration), so it
-  // is taken there only on request (PCU_CHAIN=1).
-  const bool chain = rhs_in_gram && !wide_rhs && nref == 1 && !mehrotra && !opt_no_chain &&
-                     !opt_no_fuse21 && !opt_no_fuse2s && ctx->chain_ok() &&
+  // The default iteration's solve: one refinement step done in the column space of
+  // [A|Z], one pass (kktChain).  Its dense algebra runs on the device by default on one
+  // GPU; across GPUs the host is faster (measured at 8 GPUs with the earlier two-pass
+  // chain: 1.94 against 2.04 ms per iteration), so the device is taken there only on
+  // request (PCU_CHAIN=1).  PCU_NO_FUSE21 / PCU_NO_FUSE2S select the elementwise
+  // refinement of the two-pass route below.
+  const bool colref = !inexact_newton_step && rhs_in_gram && !wide_rhs && nref == 1 &&
+                      !mehrotra && !opt_no_fuse21 && !opt_no_fuse2s;
+  const bool chain = colref && !opt_no_chain && ctx->chain_ok() &&
                      (ctx->world == 1 || opt_force_chain);
   if (inexact_newton_step) {
     // nothing to set up
-  } else if (chain) {
-    if (kktChain(v, res, upd, use_qn, mu_for_res, tau_pre, VTp.data())) return 1;
+  } else if (colref) {
+    if (kktChain(v, res, upd, use_qn, mu_for_res, tau_pre, VTp.data(), chain)) return 1;
   } else if (rhs_in_gram) {
     if (setUpKKTDiagRhs(v, use_qn, mu_for_res)) return 1;
     if (setUpKKTSystem(v, use_qn, nullptr, 1)) return 1;
@@ -1550,7 +1518,7 @@ int pcu_ip::iterate_once(int *converged) {
     }
     return 0;
   };
-  if (!chain && !inexact_newton_step) {
+  if (!colref && !inexact_newton_step) {
     // the fraction-to-boundary parameter is known before the solves (it depends on
     // the barrier only, IP.cpp:5069-5077), so the last pass of the last solve can
     // take the step statistics (not under the Mehrotra strategies, whose

@@ -69,10 +69,10 @@ __device__ __forceinline__ double gamma_sw(const IPConst &k, long long ci) {
 // device chain of the KKT solve, pcu_dense.cu -- from a constant bank that a
 // stream-ordered device-to-device copy fills from the dense kernel's output right
 // before this launch (cudaMemcpyToSymbolAsync): the same constant-cache operand either
-// way, no load in the column loops.  Layout: alpha | beta of Pass2R1F, alpha of Pass2SF.
+// way, no load in the column loops.  Layout: alpha of Pass2SVF (pcu_dense_solve).
 // (One bank per device and process: the chain is only taken while a single context
 // uses the device, pcu_ctx::chain_ok.)
-static __constant__ double pcu_chain_coef[3 * PCU_DENSE_MAXM];
+static __constant__ double pcu_chain_coef[PCU_DENSE_MAXM];
 __device__ __forceinline__ double pcu_coef(int cbank, const CoefTable &tab, int j) {
   return cbank >= 0 ? pcu_chain_coef[cbank + j] : tab.v[j];
 }
@@ -1032,15 +1032,28 @@ struct StatsF : NoStreams {
 // step statistics are taken from the step while it is still in registers, so
 // the separate 9N + 8W statistics pass disappears (one extra stream: g).
 // Traffic: Pass2F + N.   Reductions: as StatsF (sums in shared memory).
+//
+// Pass2SVF (FV = 1): the same pass as the ONLY pass of a KKT solve whose right-hand
+// side is the residual of the variables, computeKKTRes(vars, mu_rhs) (the default
+// iteration, refined in the column space of [A|Z]: pcu_dense_solve).  The bound rows
+// (IP.cpp:1417-1444) and the weighting rows (IP.cpp:1361-1389) of that residual are
+// formed from the variables instead of being read; never accumulating.
+// Traffic: reads (8 + m)N + 7W, writes 3N + 5W (+ N: A p_z).
 struct ConP2S {  // yw broadcast; the leader lane keeps the constraint's values for E
   static constexpr int ND = 1;
   double d[1];
   double sw, tw, zsw, ztw, psw, ptw, pzsw, pztw;
   __device__ __forceinline__ void zero() { d[0] = 0.0; }
 };
-struct Pass2SF : NoStreams {
+// mu_rhs (the barrier of the right-hand side) exists in Pass2SVF only: an empty base in
+// Pass2SF keeps that kernel's parameter block, and with it ptxas's code, unchanged
+template <int FV> struct Pass2SFRhs { double mu_rhs; };
+template <> struct Pass2SFRhs<0> {};
+template <int FV>
+struct Pass2SFT : NoStreams, Pass2SFRhs<FV> {
   static constexpr int SRC = 1;
-  static constexpr int REVERSE = 1;  // after Pass2R1F (upwards)
+  // Pass2SF follows Pass2R1F (upwards); Pass2SVF follows the Gram pass (downwards)
+  static constexpr int REVERSE = FV ? 0 : 1;
   static constexpr int MINB = PCU_MINB_PASS2S;
   static constexpr int NS = 22, NX = 1, NM = 2, NB = 1, NB2 = 2;
   static constexpr int SMEM = NS * PCU_TILE_THREADS * 8;
@@ -1054,13 +1067,14 @@ struct Pass2SF : NoStreams {
   static constexpr int NFIX = S_V0;  // fixed slots; the columns follow
   enum { W_CW, W_D2, W_SW, W_TW, W_ZSW, W_ZTW, W_BSW, W_BTW, W_BZSW, W_BZTW,
          W_YZW, W_YZSW, W_YZTW, W_YSW, W_YTW, NWSLOTS };
+  static constexpr int W_ZW = W_BSW;  // FV: zw takes the slot of the unread b.sw
   DVars v, b, y;
   const double *lb, *ub, *Dinv, *Cw, *d1, *d2, *g;
   ColTable V;
   CoefTable alpha;
   int cbank;  // >= 0: alpha at this offset of the constant bank (chain mode); -1: `alpha`
   int ncols;
-  int accumulate;
+  int accumulate;  // FV: 0
   double tau;
   IPConst k;
   // optional output: sum over the first nca columns (the constraint gradients) of
@@ -1072,10 +1086,10 @@ struct Pass2SF : NoStreams {
   template <class P>
   __device__ __forceinline__ void streams(P &p_) const {
     p_(d1); p_(Dinv); p_(v.x); p_(lb); p_(ub); p_(g);
-    if (k.use_lower) { p_(v.zl); p_(b.zl); }
-    if (k.use_upper) { p_(v.zu); p_(b.zu); }
+    if (k.use_lower) { p_(v.zl); if (!FV) p_(b.zl); }
+    if (k.use_upper) { p_(v.zu); if (!FV) p_(b.zu); }
     for (int j = 0; j < ncols; j++) p_(V.p[j]);
-    if (accumulate) {
+    if (!FV && accumulate) {
       p_(y.x);
       if (k.use_lower) p_(y.zl);
       if (k.use_upper) p_(y.zu);
@@ -1085,9 +1099,9 @@ struct Pass2SF : NoStreams {
   __host__ __device__ __forceinline__ void tstreams(P &p_) const {
     p_.n(S_D1, d1); p_.n(S_DINV, Dinv); p_.n(S_X, v.x); p_.n(S_LB, lb); p_.n(S_UB, ub);
     p_.n(S_G, g);
-    if (k.use_lower) { p_.n(S_ZL, v.zl); p_.n(S_BZL, b.zl); }
-    if (k.use_upper) { p_.n(S_ZU, v.zu); p_.n(S_BZU, b.zu); }
-    if (accumulate) {
+    if (k.use_lower) { p_.n(S_ZL, v.zl); if (!FV) p_.n(S_BZL, b.zl); }
+    if (k.use_upper) { p_.n(S_ZU, v.zu); if (!FV) p_.n(S_BZU, b.zu); }
+    if (!FV && accumulate) {
       p_.n(S_YX, y.x);
       if (k.use_lower) p_.n(S_YZL, y.zl);
       if (k.use_upper) p_.n(S_YZU, y.zu);
@@ -1095,8 +1109,12 @@ struct Pass2SF : NoStreams {
     for (int j = 0; j < ncols; j++) p_.n(S_V0 + j, V.p[j]);
     p_.w(W_CW, Cw); p_.w(W_D2, d2);
     p_.w(W_SW, v.sw); p_.w(W_TW, v.tw); p_.w(W_ZSW, v.zsw); p_.w(W_ZTW, v.ztw);
-    p_.w(W_BSW, b.sw); p_.w(W_BTW, b.tw); p_.w(W_BZSW, b.zsw); p_.w(W_BZTW, b.ztw);
-    if (accumulate) {
+    if (FV) {
+      p_.w(W_ZW, v.zw);
+    } else {
+      p_.w(W_BSW, b.sw); p_.w(W_BTW, b.tw); p_.w(W_BZSW, b.zsw); p_.w(W_BZTW, b.ztw);
+    }
+    if (!FV && accumulate) {
       p_.w(W_YZW, y.zw); p_.w(W_YZSW, y.zsw); p_.w(W_YZTW, y.ztw);
       p_.w(W_YSW, y.sw); p_.w(W_YTW, y.tw);
     }
@@ -1154,12 +1172,25 @@ struct Pass2SF : NoStreams {
     con.d[0] = yw;
     const double sw = src.ldw(W_SW, v.sw, ci), tw = src.ldw(W_TW, v.tw, ci);
     const double zsw = src.ldw(W_ZSW, v.zsw, ci), ztw = src.ldw(W_ZTW, v.ztw, ci);
-    double pzsw = yw - src.ldw(W_BSW, b.sw, ci);
-    double pztw = -src.ldw(W_BTW, b.tw, ci) - yw;
-    double psw = pcu_div(src.ldw(W_BZSW, b.zsw, ci) - sw * pzsw, zsw);
-    double ptw = pcu_div(src.ldw(W_BZTW, b.ztw, ci) - tw * pztw, ztw);
+    double bsw, btw, bzsw, bztw;
+    if constexpr (FV) {  // IP.cpp:1361-1389
+      const double zw = src.ldw(W_ZW, v.zw, ci);
+      bsw = (zsw - gamma_sw(k, ci)) - zw;
+      btw = (ztw - k.gamma) + zw;
+      bzsw = this->mu_rhs - sw * zsw;
+      bztw = this->mu_rhs - tw * ztw;
+    } else {
+      bsw = src.ldw(W_BSW, b.sw, ci);
+      btw = src.ldw(W_BTW, b.tw, ci);
+      bzsw = src.ldw(W_BZSW, b.zsw, ci);
+      bztw = src.ldw(W_BZTW, b.ztw, ci);
+    }
+    double pzsw = yw - bsw;
+    double pztw = -btw - yw;
+    double psw = pcu_div(bzsw - sw * pzsw, zsw);
+    double ptw = pcu_div(bztw - tw * pztw, ztw);
     double pzw = yw;
-    if (accumulate) {
+    if (!FV && accumulate) {
       pzw = src.ldw(W_YZW, y.zw, ci) + yw;
       pzsw = src.ldw(W_YZSW, y.zsw, ci) + pzsw;
       pztw = src.ldw(W_YZTW, y.ztw, ci) + pztw;
@@ -1188,11 +1219,18 @@ struct Pass2SF : NoStreams {
     for (int q = 0; q < W; q++) zl[q] = zu[q] = bzl[q] = bzu[q] = 0.0;
     if (k.use_lower) {
       src.template ld<W>(S_ZL, v.zl, i, zl);
-      src.template ld<W>(S_BZL, b.zl, i, bzl);
+      if (!FV) src.template ld<W>(S_BZL, b.zl, i, bzl);
     }
     if (k.use_upper) {
       src.template ld<W>(S_ZU, v.zu, i, zu);
-      src.template ld<W>(S_BZU, b.zu, i, bzu);
+      if (!FV) src.template ld<W>(S_BZU, b.zu, i, bzu);
+    }
+    if constexpr (FV) {  // rzl, rzu of computeKKTRes (IP.cpp:1417-1444)
+#pragma unroll
+      for (int q = 0; q < W; q++) {
+        bzl[q] = -((x[q] - l[q]) * zl[q] - k.kappa * this->mu_rhs);
+        bzu[q] = -((u[q] - x[q]) * zu[q] - k.kappa * this->mu_rhs);
+      }
     }
 #pragma unroll
     for (int q = 0; q < W; q++) {
@@ -1204,7 +1242,7 @@ struct Pass2SF : NoStreams {
       if (k.use_upper && u[q] < k.mbv)
         pzu[q] = pcu_div(bzu[q] + zu[q] * px[q], u[q] - x[q]);
     }
-    if (accumulate) {
+    if (!FV && accumulate) {
       double o[W];
       src.template ld<W>(S_YX, y.x, i, o);
 #pragma unroll
@@ -1244,6 +1282,9 @@ struct Pass2SF : NoStreams {
     acc.s[13] = 0.0;
   }
 };
+// distinct types, so that kernel names and profiles tell the two passes apart
+struct Pass2SF : Pass2SFT<0> {};
+struct Pass2SVF : Pass2SFT<1> {};
 
 // ============================================================== TrialF
 // Line-search trial point (IP.cpp:3997-4013: rx, rsw, rtw via computeStepVec)
@@ -2000,7 +2041,10 @@ struct Pass2R1F : NoStreams {
   double *d2, *d1out;
   ColTable V;
   CoefTable alpha, beta;
-  int cbank;  // >= 0: alpha | beta at this offset (+ PCU_DENSE_MAXM) of the constant bank; -1: tables
+  // always -1 (the tables): the constant-bank operand form is kept because the
+  // register allocation of this kernel depends on it (reading the tables directly
+  // makes the register-fed Pass2R1F<16> spill)
+  int cbank;
   int ncols;
   int accumulate;
   int from_vars;
