@@ -292,6 +292,26 @@ int pcu_problem_transfer_bytes(pcu_problem *prob, int64_t *h2d, int64_t *d2h);
 int pcu_problem_host_times(pcu_problem *prob, double *d2h_ms, double *user_ms,
                            double *h2d_ms);
 
+/* ParOptProblem::evalHessianDiag: h = the diagonal of the Hessian of the Lagrangian at
+   (x, z, zw), for the option use_diag_hessian, which uses diag(h) + qn_sigma in place of
+   the quasi-Newton approximation.  The optimizer calls it once after every gradient
+   evaluation, with the multipliers of that point (z: ncon host values); a non-zero return
+   counts as a failed gradient evaluation.  The first form registers it on a problem of
+   pcu_problem_create (pcu_vec handles, device memory), the second on one of
+   pcu_problem_create_host (host arrays: x in the problem's mirror, zw copied to the host,
+   h copied to the device after the call).  NULL unregisters; 1 for another kind of
+   problem.  Built-in sepquad problems have the exact diagonal already.          */
+int pcu_problem_set_hessian_diag(pcu_problem *prob, void *user,
+                                 int (*eval_hessian_diag)(void *user, pcu_vec *x,
+                                                          const double *z, pcu_vec *zw,
+                                                          pcu_vec *h));
+int pcu_problem_set_hessian_diag_host(pcu_problem *prob, void *user,
+                                      int (*eval_hessian_diag)(void *user, int n,
+                                                               const double *x,
+                                                               const double *z, int nw,
+                                                               const double *zw,
+                                                               double *h));
+
 /* MPI_Allreduce(MPI_SUM) stand-in for user callbacks that reduce their own
    partial sums (e.g. examples/rosenbrock/rosenbrock.cpp:100-117): `vals` are
    host doubles, summed over the ranks of the context in place.               */
@@ -336,7 +356,12 @@ double pcu_problem_callback_ms(pcu_problem *prob);
 pcu_ip *pcu_ip_create(pcu_problem *prob);                  /* IP.cpp:182       */
 void pcu_ip_destroy(pcu_ip *ip);
 /* ParOptOptions::setOption (ParOptOptions.h:35-37); names, defaults and ranges
-   as registered by addDefaultOptions (IP.cpp:536-727).  Unknown name -> 1.     */
+   as registered by addDefaultOptions (IP.cpp:536-727).  Unknown name -> 1.
+   use_diag_hessian (0/1) takes the problem's evalHessianDiag as the Hessian; no
+   quasi-Newton object is built and qn_type is ignored.  It runs with the monotone
+   barrier, iterative_refinement_steps = 1 and 1..32 dense constraints; begin /
+   optimize refuse it (non-zero, one "ParOpt error:" line) without the callback, with
+   use_hvec_product, sequential_linear_method or a pcu_ip_set_quasi_newton object. */
 int pcu_ip_set_option_float(pcu_ip *ip, const char *name, double value);
 int pcu_ip_set_option_int(pcu_ip *ip, const char *name, int value);
 int pcu_ip_set_option_str(pcu_ip *ip, const char *name, const char *value);

@@ -20,6 +20,14 @@ but the objective and constraint values.  `AutogradProblem` needs only `objcon(x
 -> (f, c)` in torch and takes the gradients and Hessian-vector products
 (`use_hvec_product`) from autograd.
 
+A `Problem` or `TorchProblem` subclass that defines `evalHessianDiag(x, z, zw,
+hdiag)` -- the diagonal of the Hessian of the Lagrangian, written into `hdiag` --
+can run with the option `use_diag_hessian`: the interior point then takes
+`diag(hdiag) + qn_sigma` as its Hessian in place of a quasi-Newton approximation
+(an exact Newton method where the Hessian is diagonal).  It runs with the monotone
+barrier, one refinement step and 1 to 32 dense constraints; other settings, the
+trust region and `AutogradProblem` are refused.
+
     class Model(ParOpt.TorchProblem):
         def evalObjConGradient(self, x, g, A): g.copy_(...); A[0].copy_(...)
 """

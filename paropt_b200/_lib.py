@@ -52,6 +52,9 @@ HVEC_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, c_double_p, C.c_void_p, C
                       C.c_void_p)
 
 
+HDIAG_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, c_double_p, C.c_void_p, C.c_void_p)
+
+
 class Callbacks(C.Structure):
     _fields_ = [("user", C.c_void_p), ("get_vars_and_bounds", GET_VARS_CB),
                 ("eval_obj_con", EVAL_OBJ_CB),
@@ -72,6 +75,10 @@ HOST_EVAL_GRAD_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int, c_double_p, c_doub
 HOST_WRITE_OUT_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int, C.c_int, c_double_p)
 HOST_HVEC_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int, c_double_p, c_double_p, C.c_int,
                            c_double_p, c_double_p, c_double_p)
+
+
+HOST_HDIAG_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int, c_double_p, c_double_p, C.c_int,
+                            c_double_p, c_double_p)
 
 
 class HostCallbacks(C.Structure):
@@ -165,6 +172,8 @@ SIGNATURES = {
                                              C.POINTER(C.c_int64)]),
     "pcu_problem_host_times": (C.c_int, [VP, c_double_p, c_double_p, c_double_p]),
     "pcu_problem_destroy": (None, [VP]),
+    "pcu_problem_set_hessian_diag": (C.c_int, [VP, VP, HDIAG_CB]),
+    "pcu_problem_set_hessian_diag_host": (C.c_int, [VP, VP, HOST_HDIAG_CB]),
     "pcu_ctx_allreduce_sum": (C.c_int, [VP, c_double_p, C.c_int]),
     "pcu_problem_create_sepquad_host": (VP, [VP, C.POINTER(SepQuadParams), C.c_int,
                                              C.POINTER(VP)]),

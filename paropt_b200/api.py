@@ -451,6 +451,12 @@ class Problem:
             int(use_lower), int(use_upper), C.byref(self._w), C.byref(self._cb))
         if not self.h:
             raise RuntimeError("paropt_b200: problem creation failed")
+        # ParOptProblem::evalHessianDiag: evalHessianDiag(x, z, zw, hdiag) -> fail, for the
+        # option use_diag_hessian
+        if hasattr(self, "evalHessianDiag"):
+            self._hdiag_cb = _lib.HOST_HDIAG_CB(self._eval_hdiag)
+            _check(self.lib.pcu_problem_set_hessian_diag_host(self.h, None, self._hdiag_cb),
+                   "set_hessian_diag_host")
 
     def _view(self, ptr, n):
         """numpy view of a library-owned host array (cached per address)."""
@@ -505,6 +511,17 @@ class Problem:
             traceback.print_exc()
             return 1
 
+    def _eval_hdiag(self, user, n, x, z, nw, zw, hdiag):
+        try:
+            zz = np.array([z[i] for i in range(self.ncon)])
+            fail = self.evalHessianDiag(self._view(x, n), zz, self._view(zw, nw),
+                                        self._view(hdiag, n))
+            return int(fail or 0)
+        except Exception:
+            import traceback
+            traceback.print_exc()
+            return 1
+
     def _write_output(self, user, it, n, x):
         try:
             self.writeOutput(int(it), self._view(x, n))
@@ -549,6 +566,7 @@ class TorchProblem:
         evalObjConGradient(x, g, A) -> fail          A: list of ncon tensors
         writeOutput(it, x)                           optional
         evalHvecProduct(x, z, zw, px, hvec) -> fail  optional; z: ncon host values
+        evalHessianDiag(x, z, zw, hdiag) -> fail     optional (use_diag_hessian)
         computeQuasiNewtonUpdateCorrection(x, z, zw, s, y) -> fail   optional
 
     Every vector is a float64 CUDA tensor viewing the library's own memory: fill the
@@ -605,6 +623,10 @@ class TorchProblem:
             int(use_lower), int(use_upper), C.byref(self._w), C.byref(self._cb))
         if not self.h:
             raise RuntimeError("paropt_b200: problem creation failed")
+        if hasattr(self, "evalHessianDiag"):
+            self._hdiag_cb = _lib.HDIAG_CB(self._eval_hdiag)
+            _check(self.lib.pcu_problem_set_hessian_diag(self.h, None, self._hdiag_cb),
+                   "set_hessian_diag")
 
     def _vec(self, h):
         """Zero-copy tensor view of a pcu_vec, cached by handle and device pointer: the
@@ -705,6 +727,11 @@ class TorchProblem:
         zz = np.array([z[i] for i in range(self.ncon)])
         return self._call(lambda: self.evalHvecProduct(
             self._vec(x), zz, self._vec(zw), self._vec(px), self._vec(hvec)))
+
+    def _eval_hdiag(self, user, x, z, zw, hdiag):
+        zz = np.array([z[i] for i in range(self.ncon)])
+        return self._call(lambda: self.evalHessianDiag(
+            self._vec(x), zz, self._vec(zw), self._vec(hdiag)))
 
     def _qn_correction(self, user, x, z, zw, s, y):
         zz = np.array([z[i] for i in range(self.ncon)])

@@ -60,6 +60,7 @@ const OptEntry OPTIONS[] = {
     OPT_I(write_output_frequency, 0, 1000000),
     OPT_I(history_level, 0, 2),
     OPT_I(use_hvec_product, 0, 1),
+    OPT_I(use_diag_hessian, 0, 1),
     OPT_I(use_qn_gmres_precon, 0, 1),
     OPT_I(gmres_subspace_size, 0, 1000),
     OPT_F(nk_switch_tol, 0.0, 1e20),
@@ -546,7 +547,7 @@ int pcu_ip_comp(pcu_ip *ip, double *comp) {
 }
 
 int pcu_ip_setup_kkt_diag(pcu_ip *ip, int use_qn) {
-  if (ip->ensure_qn()) return 1;
+  if (ip->diagHessianRefused() || ip->ensure_qn()) return 1;
   if (ip->setUpKKTDiagSystem(ip->variables, use_qn, 0)) return 1;
   return ip->setUpKKTSystem(ip->variables, 0, nullptr);
 }
@@ -565,7 +566,7 @@ int pcu_ip_kkt_step(pcu_ip *ip, int res, int step, int use_qn) {
 int pcu_ip_add_kkt_res_step(pcu_ip *ip, int step, int res) {
   Vars *s = bundle(ip, step), *r = bundle(ip, res);
   if (!r || !s) return 1;
-  if (ip->ensure_qn()) return 1;
+  if (ip->diagHessianRefused() || ip->ensure_qn()) return 1;
   ip->refresh_penalties();
   std::vector<double> dots;
   if (step_dots(ip, *s, dots)) return 1;
@@ -576,7 +577,7 @@ int pcu_ip_add_kkt_res_step(pcu_ip *ip, int step, int res) {
 int pcu_ip_kkt_solve(pcu_ip *ip, int res, int step, int on_device) {
   Vars *r = bundle(ip, res), *s = bundle(ip, step);
   if (!r || !s) return 1;
-  if (ip->ensure_qn()) return 1;
+  if (ip->diagHessianRefused() || ip->ensure_qn()) return 1;
   if (on_device && !ip->ctx->chain_ok()) return 1;
   ip->refresh_penalties();
   const int m = ip->ncon + (ip->qn ? ip->qn->size() : 0);

@@ -396,7 +396,8 @@ pcu_ip::~pcu_ip() {
   Vars *all[4] = {&variables, &residual, &update, &refine};
   for (auto vs : all)
     for (int i = 0; i < 8; i++) pcu_vec_destroy(vs->v[i]);
-  pcu_vec *single[] = {lb, ub, g, Dinv, Cw, d1, d2, t1, s_qn, y_qn, rx, rsw, rtw, gaz, apz1, apz2};
+  pcu_vec *single[] = {lb, ub, g, Dinv, Cw, d1, d2, t1, s_qn, y_qn, rx, rsw, rtw, gaz, apz1, apz2,
+                       hdiag};
   for (auto v : single) pcu_vec_destroy(v);
   for (auto v : Ac) pcu_vec_destroy(v);
   for (auto v : gmres_W) pcu_vec_destroy(v);
@@ -508,6 +509,13 @@ int pcu_ip::norm_type_id() const {
 
 int pcu_ip::ensure_qn() {  // IP.cpp:263-290
   if (qn_external) return qn ? 0 : 1;  // supplied through pcu_ip_set_quasi_newton
+  if (opt.use_diag_hessian) {  // the problem's diagonal is the Hessian: no quasi-Newton object
+    if (qn) delete qn;
+    qn = nullptr;
+    qn_built_type.clear();
+    qn_built_size = -1;
+    return 0;
+  }
   if (qn && qn_built_type == opt.qn_type && qn_built_size == opt.qn_subspace_size) {
     qn->damped = (opt.qn_update_type == "damped_update");
     qn->diag_yts_over_sts = (opt.qn_diag_type == "yts_over_sts");
@@ -624,8 +632,14 @@ int pcu_ip::evalObjConGradient(pcu_vec *x, int same_point) {
   prob->same_point_hint = same_point;
   gaz_valid = 0;
   int fail = prob->evalObjConGradient(x, g, Ac.data());
-  prob->same_point_hint = 0;
   ngeval++;
+  // use_diag_hessian: the diagonal at the point the gradient callback just saw, with
+  // that point's multipliers; a failure counts as a failed gradient evaluation
+  if (!fail && opt.use_diag_hessian) {
+    prob->same_point_hint = 1;
+    fail = prob->evalHessianDiag(x, variables.z.data(), variables.v[PCU_ZW], hdiag);
+  }
+  prob->same_point_hint = 0;
   if (cb_end()) return 1;
   return fail;
 }
@@ -737,6 +751,40 @@ void pcu_ip::apz_done(int accumulate, double *target) {
 }
 
 // --------------------------------------------------------------- residuals
+// use_diag_hessian: the Hessian term of addKKTResStep, rx -= h p_x (IP.cpp:1464), after
+// ResF has formed the rest of the row, with the norms of rx taken again (ResF's sums 3 and
+// maximum 0).  Only the stand-alone residual of a step reaches it (pcu_ip_add_kkt_res_step):
+// the optimizer's route with this option refines in the column space of [A|Z].
+// Traffic: reads 3N, writes N.
+struct HessDiagResF : NoStreams {
+  static constexpr int NS = 2, NX = 1, NM = 0, NB = 0;
+  typedef Acc<NS, NX, NM> AccT;
+  typedef Con0 Con;
+  struct Elem {};
+  const double *h, *px;
+  double *rx;
+  template <int W>
+  __device__ __forceinline__ void A(long long, const double (&)[W], Elem (&)[W],
+                                    double (&)[W][1], AccT *) const {}
+  __device__ __forceinline__ void B(long long, const double (&)[1], Con &, AccT &) const {}
+  template <int W>
+  __device__ __forceinline__ void C(long long i, const double (&)[W], const Elem (&)[W],
+                                    const Con &, AccT &acc) const {
+    double hv[W], p[W], r[W];
+    ldv<W>(h, i, hv);
+    ldv<W>(px, i, p);
+    ldv<W>(rx, i, r);
+#pragma unroll
+    for (int q = 0; q < W; q++) {
+      r[q] = fma(-hv[q], p[q], r[q]);
+      acc.x[0] = fmax(acc.x[0], fabs(r[q]));
+      acc.s[0] += fabs(r[q]);
+      acc.s[1] = fma(r[q], r[q], acc.s[1]);
+    }
+    stv<W>(rx, i, r);
+  }
+};
+
 int pcu_ip::computeKKTRes(Vars &vars, double mu, Vars &res, Vars *step,
                           const double *ATp, const double *ZTp, int store) {
   ResF f;
@@ -787,6 +835,22 @@ int pcu_ip::computeKKTRes(Vars &vars, double mu, Vars &res, Vars *step,
   memcpy(res_sums, out, sizeof(res_sums));
   memcpy(res_max, out + ResF::NS, sizeof(res_max));
   memcpy(res_min, out + ResF::NS + ResF::NX, sizeof(res_min));
+  if (step && opt.use_diag_hessian && !res_skip_hessian) {
+    if (!store) return 1;
+    HessDiagResF fh;
+    fh.h = hdiag->d;
+    fh.px = step->v[PCU_X]->d;
+    fh.rx = res.v[PCU_X]->d;
+    WDesc w0;
+    memset(&w0, 0, sizeof(w0));
+    RedBuf rbh = ctx->redbuf(HessDiagResF::NS, HessDiagResF::NX, 0);
+    if (launch_tile(ctx, fh, nvars, w0, rbh)) return 1;
+    double oh[3];
+    if (ctx->fetch(oh)) return 1;
+    res_max[0] = oh[2];
+    if (f.norm_type == 1) res_sums[3] = oh[0];
+    else if (f.norm_type == 2) res_sums[3] = oh[1];
+  }
   res_mu = mu;
   res_has_step = step ? 1 : 0;
   denseResidual(vars, mu, res, step, ATp);

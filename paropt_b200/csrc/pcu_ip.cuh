@@ -42,6 +42,9 @@ struct IPOptions {
   int history_level = 1;  // 0 none, 1 scalars, 2 + state checksums (one extra pass)
   // inexact-Newton GMRES path (IP.cpp:593-611, 639, 646, 668)
   int use_hvec_product = 0;
+  // the problem's diagonal Hessian of the Lagrangian (evalHessianDiag) in place of the
+  // quasi-Newton approximation (IP.cpp:1464, 1842, 3811, 4458)
+  int use_diag_hessian = 0;
   int use_qn_gmres_precon = 1;
   int gmres_subspace_size = 0;
   double nk_switch_tol = 1e-3;
@@ -138,6 +141,7 @@ struct pcu_ip {
   pcu_vec *d1 = nullptr, *d2 = nullptr, *t1 = nullptr;  // KKT-solve scratch
   pcu_vec *s_qn = nullptr, *y_qn = nullptr;
   pcu_vec *rx = nullptr, *rsw = nullptr, *rtw = nullptr;  // line-search trial
+  pcu_vec *hdiag = nullptr;  // use_diag_hessian: h of the last gradient evaluation
   // g - A z at the current point, written by the last update pass (ncon >= 3): the first
   // pass of the next KKT solve reads it instead of g and the ncon constraint gradients
   pcu_vec *gaz = nullptr;
@@ -185,6 +189,7 @@ struct pcu_ip {
   int stats_ready = 0;        // Pass2SF / Pass2SVF left the step statistics in stats_out
   double stats_tau_used = 0.0;
   double stats_out[32];
+  double stats_hp2 = 0.0;     // sum h p^2 of the last Pass2SVHF (use_diag_hessian)
   int opt_no_wide = 0;        // debugging: more than 32 columns stay on the register-fed pass 2
   int opt_no_fuse21 = 0;      // debugging: refine elementwise, pass 2 and the next pass 1 separate
   // residual statistics of the NEXT iteration taken by the update passes (ResF layout)
@@ -278,6 +283,7 @@ struct pcu_ip {
   int evalHvecProduct(pcu_vec *px, pcu_vec *hvec);
   int initLeastSquaresMultipliers();
   int initAffineStepMultipliers();
+  int diagHessianRefused();  // use_diag_hessian with a route it does not cover: prints why
   int begin();
   int iterate_once(int *converged);
   int snapshot(int k, double comp, double max_prime, double max_dual,

@@ -35,20 +35,29 @@ enum { BS_MONOTONE = 0, BS_MEHROTRA = 1, BS_MPC = 2, BS_COMP_FRACTION = 3 };
 // IP.cpp:1832-1930 (diagonal + Ew factor; G follows in setUpKKTSystem)
 int pcu_ip::setUpKKTDiagSystem(Vars &vars, int use_qn, int identity) {
   pass1_ready = 0;
-  DiagF f;
-  f.v = vars.dv();
-  f.lb = lb->d;
-  f.ub = ub->d;
-  f.Dinv = Dinv->d;
-  f.Cw = Cw->d;
-  double b0 = 0.0;
-  if (qn && use_qn) b0 = qn->b0;
-  b0_used = b0;
-  f.b0sig = b0 + opt.qn_sigma;
-  f.identity = identity;
-  f.small_ = 1e-4;
-  f.k = kconst();
-  return launch_tile(ctx, f, nvars, wd, NO_RED);
+  auto launch = [&](auto f) -> int {
+    f.v = vars.dv();
+    f.lb = lb->d;
+    f.ub = ub->d;
+    f.Dinv = Dinv->d;
+    f.Cw = Cw->d;
+    double b0 = 0.0;
+    if (qn && use_qn) b0 = qn->b0;
+    b0_used = b0;
+    f.b0sig = b0 + opt.qn_sigma;
+    f.identity = identity;
+    f.small_ = 1e-4;
+    f.k = kconst();
+    return launch_tile(ctx, f, nvars, wd, NO_RED);
+  };
+  // use_diag_hessian: diag(h) is the Hessian where the loop takes one (use_qn), as the
+  // quasi-Newton b0 is: D0 = h + sigma + bound terms
+  if (opt.use_diag_hessian && use_qn && !identity) {
+    DiagHF f;
+    f.h = hdiag->d;
+    return launch(f);
+  }
+  return launch(DiagF());
 }
 
 // setUpKKTDiagSystem + the right-hand side (d1, d2) of the iteration's first
@@ -56,32 +65,39 @@ int pcu_ip::setUpKKTDiagSystem(Vars &vars, int use_qn, int identity) {
 // (setUpKKTSystem with_rhs).
 int pcu_ip::setUpKKTDiagRhs(Vars &vars, int use_qn, double mu) {
   pass1_ready = 0;
-  DiagRhsF f;
-  f.v = vars.dv();
-  f.lb = lb->d;
-  f.ub = ub->d;
-  f.g = g->d;
-  f.Dinv = Dinv->d;
-  f.Cw = Cw->d;
-  f.d1 = d1->d;
-  f.d2 = d2->d;
-  f.ncon = ncon;
-  for (int j = 0; j < ncon; j++) {
-    f.Acol.p[j] = Ac[j]->d;
-    f.z.v[j] = vars.z[j];
+  auto launch = [&](auto f) -> int {
+    f.v = vars.dv();
+    f.lb = lb->d;
+    f.ub = ub->d;
+    f.g = g->d;
+    f.Dinv = Dinv->d;
+    f.Cw = Cw->d;
+    f.d1 = d1->d;
+    f.d2 = d2->d;
+    f.ncon = ncon;
+    for (int j = 0; j < ncon; j++) {
+      f.Acol.p[j] = Ac[j]->d;
+      f.z.v[j] = vars.z[j];
+    }
+    if (gaz_valid && &vars == &variables) {
+      // g - A z of this very point was left by the last update pass
+      f.g = gaz->d;
+      f.ncon = 0;
+    }
+    double b0 = 0.0;
+    if (qn && use_qn) b0 = qn->b0;
+    b0_used = b0;
+    f.b0sig = b0 + opt.qn_sigma;
+    f.mu = mu;
+    f.k = kconst();
+    return launch_tile(ctx, f, nvars, wd, NO_RED);
+  };
+  if (opt.use_diag_hessian && use_qn) {  // D0 = h + sigma + bound terms
+    DiagRhsHF f;
+    f.h = hdiag->d;
+    return launch(f);
   }
-  if (gaz_valid && &vars == &variables) {
-    // g - A z of this very point was left by the last update pass
-    f.g = gaz->d;
-    f.ncon = 0;
-  }
-  double b0 = 0.0;
-  if (qn && use_qn) b0 = qn->b0;
-  b0_used = b0;
-  f.b0sig = b0 + opt.qn_sigma;
-  f.mu = mu;
-  f.k = kconst();
-  return launch_tile(ctx, f, nvars, wd, NO_RED);
+  return launch(DiagRhsF());
 }
 
 // ----------------------------------------------------------- setUpKKTSystem
@@ -590,23 +606,37 @@ int pcu_ip::kktChain(Vars &vars, Vars &b, Vars &y, int use_qn, double mu, double
     pcu_dense_host(h, o, Sg.data());
   }
   // ---- the one pass: the refined step + the step statistics
-  Pass2SVF fs;
-  fs.v = vars.dv(); fs.b = b.dv(); fs.y = y.dv();
-  fs.lb = lb->d; fs.ub = ub->d; fs.Dinv = Dinv->d; fs.Cw = Cw->d;
-  fs.d1 = d1->d; fs.d2 = d2->d; fs.g = g->d;
-  fs.V = V;
-  fs.cbank = on_device ? 0 : -1;
-  if (!on_device)
-    for (int j = 0; j < m; j++) fs.alpha.v[j] = h[o.coef + j];
-  fs.ncols = m;
-  fs.accumulate = 0; fs.tau = tau; fs.mu_rhs = mu; fs.k = kconst();
-  fs.apz = apz_target(0, true);
-  fs.nca = ncon;
-  RedBuf rb = ctx->redbuf(Pass2SVF::NS, Pass2SVF::NX, Pass2SVF::NM);
-  if (launch_tile(ctx, fs, nvars, wd, rb)) return 1;
-  apz_done(0, fs.apz);
-  PCU_CUDA_OK(cudaEventRecord(evs[ev_cur].k1, ctx->stream));
-  if (ctx->fetch(stats_out)) return 1;
+  auto pass = [&](auto fs) -> int {
+    fs.v = vars.dv(); fs.b = b.dv(); fs.y = y.dv();
+    fs.lb = lb->d; fs.ub = ub->d; fs.Dinv = Dinv->d; fs.Cw = Cw->d;
+    fs.d1 = d1->d; fs.d2 = d2->d; fs.g = g->d;
+    fs.V = V;
+    fs.cbank = on_device ? 0 : -1;
+    if (!on_device)
+      for (int j = 0; j < m; j++) fs.alpha.v[j] = h[o.coef + j];
+    fs.ncols = m;
+    fs.accumulate = 0; fs.tau = tau; fs.mu_rhs = mu; fs.k = kconst();
+    fs.apz = apz_target(0, true);
+    fs.nca = ncon;
+    typedef decltype(fs) F;
+    RedBuf rb = ctx->redbuf(F::NS, F::NX, F::NM);
+    if (launch_tile(ctx, fs, nvars, wd, rb)) return 1;
+    apz_done(0, fs.apz);
+    PCU_CUDA_OK(cudaEventRecord(evs[ev_cur].k1, ctx->stream));
+    return ctx->fetch(stats_out);
+  };
+  if (opt.use_diag_hessian) {
+    Pass2SVHF fs;
+    fs.h = hdiag->d;
+    if (pass(fs)) return 1;
+    // sum h p^2 follows the 22 sums of StatsF's layout: take it out, so that the maximum
+    // and the minima sit where stepStats reads them
+    const int ns = StatsF::NS;
+    stats_hp2 = stats_out[ns];
+    for (int i = ns; i < ns + StatsF::NX + StatsF::NM; i++) stats_out[i] = stats_out[i + 1];
+  } else if (pass(Pass2SVF())) {
+    return 1;
+  }
   stats_ready = 1;
   stats_tau_used = tau;
   // ---- host mirrors of what the dense algebra produced
@@ -1076,6 +1106,9 @@ int pcu_ip::scaleAndMerit(Vars &v, Vars &upd, double tau, double comp,
   double sums[StatsF::NS], mins[2];
   double alpha_x = 1.0, alpha_z = 1.0, m0 = 0.0, dm0 = 0.0, pnorm2 = 0.0;
   int ceq_step = 0;
+    // (stepStats consumes the statistics of the pass that formed the step)
+    const bool hp2_ready = stats_ready && stats_tau_used == tau;
+    const double hp2 = stats_hp2;
     if (stepStats(v, upd, tau, sums, mins)) return 1;
     alpha_x = mins[0];
     alpha_z = mins[1];
@@ -1140,7 +1173,15 @@ int pcu_ip::scaleAndMerit(Vars &v, Vars &upd, double tau, double comp,
     const double infeas_proj = infeas > 0.0 ? (pdense_infeas + psparse) / infeas : 0.0;
     // p^T B p through the compact form (IP.cpp:3820-3821)
     double pTBp = 0.0;
-    if (qn && !slm) {
+    if (opt.use_diag_hessian) {
+      // the compact form's expression with B = diag(h): sum h p^2, taken by the pass that
+      // formed the step (Pass2SVHF); a step from elsewhere has no such sum
+      if (!hp2_ready) {
+        fprintf(stderr, "ParOpt error: use_diag_hessian: this step has no p^T diag(h) p\n");
+        return 1;
+      }
+      pTBp = 0.5 * alpha_x * alpha_x * hp2;
+    } else if (qn && !slm) {
       double v2 = qn->b0 * sums[17];
       const int q = qn->size();
       if (q > 0) {
@@ -1198,12 +1239,36 @@ int pcu_ip::scaleAndMerit(Vars &v, Vars &upd, double tau, double comp,
     return 0;
 }
 
+// --------------------------------------------------------- use_diag_hessian
+// The diagonal Hessian runs on the default iteration's route only: monotone barrier,
+// one refinement step done in the column space of [A|Z] (kktChain) with 1 <= ncon <= 32
+// dense constraints, any starting-point strategy.  Everything else is refused here
+// rather than run with a Hessian term missing.
+int pcu_ip::diagHessianRefused() {
+  if (!opt.use_diag_hessian) return 0;
+  const char *why = nullptr;
+  if (!prob->hasHessianDiag()) why = "the problem has no evalHessianDiag";
+  else if (opt.use_hvec_product) why = "use_hvec_product is not available with it";
+  else if (qn_external) why = "a quasi-Newton object set by setQuasiNewton is not used with it";
+  else if (opt.sequential_linear_method) why = "sequential_linear_method is not available with it";
+  else if (opt.barrier_strategy != "monotone") why = "it needs barrier_strategy = monotone";
+  else if (opt.iterative_refinement_steps != 1) why = "it needs iterative_refinement_steps = 1";
+  else if (ncon < 1 || ncon > 32) why = "it needs 1 to 32 dense constraints";
+  if (why) {
+    if (ctx->rank == 0) fprintf(stderr, "ParOpt error: use_diag_hessian: %s\n", why);
+    return 1;
+  }
+  if (!hdiag) hdiag = pcu_vec_create(ctx, nvars);
+  return hdiag ? 0 : 1;
+}
+
 // -------------------------------------------------------------------- begin
 // Everything ParOptInteriorPoint::optimize does before its major loop
 // (IP.cpp:4399-4606).
 int pcu_ip::begin() {
   gaz_valid = 0;
   apz_state = 0;
+  if (diagHessianRefused()) return 1;
   if (ensure_qn()) return 1;
   refresh_penalties();
   if (!opt.output_file.empty() && !outfp && ctx->rank == 0) {
@@ -1224,7 +1289,7 @@ int pcu_ip::begin() {
   status = 0;
   history.clear();
   times.clear();
-  if (!opt.sequential_linear_method && !qn) {
+  if (!opt.sequential_linear_method && !qn && !opt.use_diag_hessian) {
     if (ctx->rank == 0)
       fprintf(stderr,
               "ParOpt Error: Must use a sequential linear method if no "
@@ -1271,10 +1336,13 @@ int pcu_ip::iterate_once(int *converged) {
   PCU_CUDA_OK(cudaEventRecord(evs[ev_cur].k0, ctx->stream));
   PCU_CUDA_OK(cudaEventRecord(evs[ev_cur].k1, ctx->stream));
 
+  // (use_diag_hessian: diag(h) stands where the quasi-Newton object does; its "reset"
+  // changes nothing, h comes from the problem, and is reported as the object's is)
+  const bool hess_obj = qn || opt.use_diag_hessian;
   int qn_hessian_reset = 0;
-  if (qn && !slm) {
+  if (hess_obj && !slm) {
     if (k > 0 && k % opt.hessian_reset_freq == 0 && uq) {
-      qn->reset();
+      if (qn) qn->reset();
       qn_hessian_reset = 1;
     }
   }
@@ -1478,6 +1546,14 @@ int pcu_ip::iterate_once(int *converged) {
                       !mehrotra && !opt_no_fuse21 && !opt_no_fuse2s;
   const bool chain = colref && !opt_no_chain && ctx->chain_ok() &&
                      (ctx->world == 1 || opt_force_chain);
+  if (opt.use_diag_hessian && (!colref || !hdiag || qn)) {
+    // (the other routes would miss the Hessian term of their refinement residual; the
+    // option has to be set before begin)
+    if (ctx->rank == 0)
+      fprintf(stderr, "ParOpt error: use_diag_hessian: this iteration is not on the route "
+                      "of the column-space refinement, or the option was set after begin\n");
+    return 1;
+  }
   if (inexact_newton_step) {
     // nothing to set up
   } else if (colref) {
@@ -1883,17 +1959,23 @@ int pcu_ip::iterate_once(int *converged) {
         line_fail = LS_NO_IMPROVEMENT;
     } else {
       if (dm0 >= 0.0) {  // IP.cpp:5130-5173
-        if (qn) {
+        if (hess_obj) {
           qn_hessian_reset = 1;
-          qn->reset();
+          if (qn) qn->reset();
         }
         if (computeKKTRes(v, barrier_param, res, nullptr, nullptr, nullptr)) return 1;
         computeResNorm(res, &max_prime, &max_dual, &max_infeas, &res_norm);
         diagonal_qn_step = 1;
         use_qn = 1;
-        if (setUpKKTDiagSystem(v, use_qn, 0)) return 1;
-        if (setUpKKTSystem(v, use_qn, nullptr)) return 1;
-        if (kkt_with_refinement(barrier_param, true)) return 1;
+        if (opt.use_diag_hessian) {
+          // the same solve on the route this option runs on (its refinement residual
+          // carries h; the two-pass route's would not)
+          if (kktChain(v, res, upd, use_qn, barrier_param, tau, VTp.data(), chain)) return 1;
+        } else {
+          if (setUpKKTDiagSystem(v, use_qn, 0)) return 1;
+          if (setUpKKTSystem(v, use_qn, nullptr)) return 1;
+          if (kkt_with_refinement(barrier_param, true)) return 1;
+        }
         if (scale_and_merit(0)) return 1;
         ls.dm0_prev = dm0;
       }
@@ -1958,9 +2040,9 @@ int pcu_ip::iterate_once(int *converged) {
   ls.alpha_xprev = alpha_x;
   ls.alpha_zprev = alpha_z;
   ls.last_pnorm2 = pnorm2;
-  if (qn && uq && (line_fail & LS_FAILURE)) {
+  if (hess_obj && uq && (line_fail & LS_FAILURE)) {
     qn_hessian_reset = 1;
-    qn->reset();
+    if (qn) qn->reset();
   }
   std::string info;
   if (gmres_iters != 0) info += "iNK" + std::to_string(gmres_iters) + " ";

@@ -340,7 +340,15 @@ typedef ResFT<-1, -1> ResF;
 // Aw^T).  identity != 0 gives the matrices of initLeastSquaresMultipliers
 // (IP.cpp:5418-5431): Dinv = 1, Cdiag = small.
 // Traffic: reads 5N + 4W, writes N + W.
-struct DiagF : NoStreams {
+//
+// HD = 1 (use_diag_hessian): the Hessian block is diag(h) + sigma, the problem's
+// diagonal (evalHessianDiag) in place of b0 + Z M Z^T; b0sig is then sigma alone.
+// One more N-stream: reads 6N + 4W.  The h pointer exists in the HD = 1 types only, so
+// the HD = 0 kernels keep their parameter blocks and their code.
+template <int HD> struct HessDiagPtr { const double *h; };
+template <> struct HessDiagPtr<0> {};
+template <int HD>
+struct DiagFT : NoStreams, HessDiagPtr<HD> {
   static constexpr int NS = 0, NX = 0, NM = 0, NB = 1;
   typedef Acc<NS, NX, NM> AccT;
   typedef Con0 Con;
@@ -359,6 +367,7 @@ struct DiagF : NoStreams {
       p_(v.x); p_(lb); p_(ub);
       if (k.use_lower) p_(v.zl);
       if (k.use_upper) p_(v.zu);
+      if constexpr (HD) p_(this->h);
     }
   }
 
@@ -370,7 +379,7 @@ struct DiagF : NoStreams {
 #pragma unroll
       for (int q = 0; q < W; q++) d[q] = 1.0;
     } else {
-      double x[W], l[W], u[W], zl[W], zu[W];
+      double x[W], l[W], u[W], zl[W], zu[W], hv[W];
       ldv<W>(v.x, i, x);
       ldv<W>(lb, i, l);
       ldv<W>(ub, i, u);
@@ -378,9 +387,11 @@ struct DiagF : NoStreams {
       for (int q = 0; q < W; q++) zl[q] = zu[q] = 0.0;
       if (k.use_lower) ldv<W>(v.zl, i, zl);
       if (k.use_upper) ldv<W>(v.zu, i, zu);
+      if constexpr (HD) ldv<W>(this->h, i, hv);
 #pragma unroll
       for (int q = 0; q < W; q++) {
         double t = b0sig;
+        if constexpr (HD) t = hv[q] + b0sig;
         if (k.use_lower && l[q] > -k.mbv) t += zl[q] / (x[q] - l[q]);
         if (k.use_upper && u[q] < k.mbv) t += zu[q] / (u[q] - x[q]);
         d[q] = 1.0 / t;
@@ -401,6 +412,9 @@ struct DiagF : NoStreams {
                                     const Elem (&)[W], const Con &,
                                     AccT &) const {}
 };
+// distinct types, so that kernel names and profiles tell the two apart
+struct DiagF : DiagFT<0> {};
+struct DiagHF : DiagFT<1> {};
 
 // ============================================================== BlockFactorF / BlockApplyF
 // ParOptQuasiDefBlockMat with nwblock = 1 as a stand-alone object (SM.cpp:41-224):
@@ -484,10 +498,13 @@ struct BlockApplyF : NoStreams {
 // [A|Z]^T t1 then ride along in the Gram pass as one more column (pcu_gram.cu),
 // so the first solve of an iteration has no pass 1 of its own.
 // Traffic: reads (6 + c)N + 5W, writes 2N + 2W.
-struct DiagRhsF : NoStreams {
+// HD = 1 (DiagRhsHF, use_diag_hessian): c = h_i + sigma, as DiagFT<1>; reads (7 + c)N.
+template <int HD>
+struct DiagRhsFT : NoStreams, HessDiagPtr<HD> {
   static constexpr int SRC = 1;
   static constexpr int NS = 0, NX = 0, NM = 0, NB = 2, HASP = 1;
-  enum { S_X, S_LB, S_UB, S_G, S_ZL, S_ZU, S_A0 };
+  enum { S_X, S_LB, S_UB, S_G, S_ZL, S_ZU, S_H };
+  static constexpr int S_A0 = S_H + HD;
   static constexpr int NFIX = S_A0;  // fixed slots; the columns follow
   static constexpr int TROWS = 512;
   enum { W_ZW, W_SW, W_TW, W_ZSW, W_ZTW, NWSLOTS };
@@ -508,6 +525,7 @@ struct DiagRhsF : NoStreams {
     p_(v.x); p_(lb); p_(ub); p_(g);
     if (k.use_lower) p_(v.zl);
     if (k.use_upper) p_(v.zu);
+    if constexpr (HD) p_(this->h);
     for (int j = 0; j < ncon; j++) p_(Acol.p[j]);
   }
   template <class P>
@@ -515,6 +533,7 @@ struct DiagRhsF : NoStreams {
     p_.n(S_X, v.x); p_.n(S_LB, lb); p_.n(S_UB, ub); p_.n(S_G, g);
     if (k.use_lower) p_.n(S_ZL, v.zl);
     if (k.use_upper) p_.n(S_ZU, v.zu);
+    if constexpr (HD) p_.n(S_H, this->h);
     for (int j = 0; j < ncon; j++) p_.n(S_A0 + j, Acol.p[j]);
     p_.w(W_ZW, v.zw); p_.w(W_SW, v.sw); p_.w(W_TW, v.tw); p_.w(W_ZSW, v.zsw);
     p_.w(W_ZTW, v.ztw);
@@ -536,6 +555,8 @@ struct DiagRhsF : NoStreams {
     for (int q = 0; q < W; q++) zl[q] = zu[q] = 0.0;
     if (k.use_lower) src.template ld<W>(S_ZL, v.zl, i, zl);
     if (k.use_upper) src.template ld<W>(S_ZU, v.zu, i, zu);
+    double hv[W];
+    if constexpr (HD) src.template ld<W>(S_H, this->h, i, hv);
 #pragma unroll
     for (int q = 0; q < W; q++) d[q] = (zl[q] - zu[q]) - gv[q];
     for (int j = 0; j < ncon; j++) {
@@ -548,6 +569,7 @@ struct DiagRhsF : NoStreams {
     for (int q = 0; q < W; q++) {
       const double dl = x[q] - l[q], du = u[q] - x[q];
       double c = b0sig;                           // IP.cpp:1864-1910
+      if constexpr (HD) c = hv[q] + b0sig;
       double t = fma(coef[q], con.d[0], d[q]);    // rx
       if (k.use_lower && l[q] > -k.mbv) {
         const double rl = pcu_rcp(dl);
@@ -585,6 +607,8 @@ struct DiagRhsF : NoStreams {
   __device__ __forceinline__ void C(const S &, long long, const double (&)[W],
                                     const Elem (&)[W], const Con &, AT &) const {}
 };
+struct DiagRhsF : DiagRhsFT<0> {};
+struct DiagRhsHF : DiagRhsFT<1> {};
 
 // ============================================================== MehrotraCorrF
 // addMehrotraCorrectorResidual (IP.cpp:1729-1789): second-order terms of the
@@ -1039,6 +1063,11 @@ struct StatsF : NoStreams {
 // (IP.cpp:1417-1444) and the weighting rows (IP.cpp:1361-1389) of that residual are
 // formed from the variables instead of being read; never accumulating.
 // Traffic: reads (8 + m)N + 7W, writes 3N + 5W (+ N: A p_z).
+//
+// Pass2SVHF (FV = 1, HD = 1; use_diag_hessian): also reads h and adds one sum,
+// s[22] = sum h p^2, the curvature term of the merit derivative (p^T B p with
+// B = diag(h)).  h is read, not recovered from Dinv: 1/Dinv - sigma - bound terms
+// cancels where the bound terms dominate.  Reads (9 + m)N + 7W.
 struct ConP2S {  // yw broadcast; the leader lane keeps the constraint's values for E
   static constexpr int ND = 1;
   double d[1];
@@ -1049,13 +1078,14 @@ struct ConP2S {  // yw broadcast; the leader lane keeps the constraint's values 
 // Pass2SF keeps that kernel's parameter block, and with it ptxas's code, unchanged
 template <int FV> struct Pass2SFRhs { double mu_rhs; };
 template <> struct Pass2SFRhs<0> {};
-template <int FV>
-struct Pass2SFT : NoStreams, Pass2SFRhs<FV> {
+template <int FV, int HD = 0>
+struct Pass2SFT : NoStreams, Pass2SFRhs<FV>, HessDiagPtr<HD> {
+  static_assert(FV || !HD, "the diagonal Hessian runs on the variables' right-hand side");
   static constexpr int SRC = 1;
   // Pass2SF follows Pass2R1F (upwards); Pass2SVF follows the Gram pass (downwards)
   static constexpr int REVERSE = FV ? 0 : 1;
   static constexpr int MINB = PCU_MINB_PASS2S;
-  static constexpr int NS = 22, NX = 1, NM = 2, NB = 1, NB2 = 2;
+  static constexpr int NS = 22 + HD, NX = 1, NM = 2, NB = 1, NB2 = 2;
   static constexpr int SMEM = NS * PCU_TILE_THREADS * 8;
   typedef AccS<NS, NX, NM> AccT;
   typedef ConP2S Con;
@@ -1063,7 +1093,8 @@ struct Pass2SFT : NoStreams, Pass2SFRhs<FV> {
     double d1, dinv;
   };
   // staged slots (tma_tile_kernel): N-streams, then the columns; W-streams
-  enum { S_D1, S_DINV, S_X, S_LB, S_UB, S_G, S_ZL, S_BZL, S_ZU, S_BZU, S_YX, S_YZL, S_YZU, S_V0 };
+  enum { S_D1, S_DINV, S_X, S_LB, S_UB, S_G, S_ZL, S_BZL, S_ZU, S_BZU, S_YX, S_YZL, S_YZU, S_H };
+  static constexpr int S_V0 = S_H + HD;
   static constexpr int NFIX = S_V0;  // fixed slots; the columns follow
   enum { W_CW, W_D2, W_SW, W_TW, W_ZSW, W_ZTW, W_BSW, W_BTW, W_BZSW, W_BZTW,
          W_YZW, W_YZSW, W_YZTW, W_YSW, W_YTW, NWSLOTS };
@@ -1088,6 +1119,7 @@ struct Pass2SFT : NoStreams, Pass2SFRhs<FV> {
     p_(d1); p_(Dinv); p_(v.x); p_(lb); p_(ub); p_(g);
     if (k.use_lower) { p_(v.zl); if (!FV) p_(b.zl); }
     if (k.use_upper) { p_(v.zu); if (!FV) p_(b.zu); }
+    if constexpr (HD) p_(this->h);
     for (int j = 0; j < ncols; j++) p_(V.p[j]);
     if (!FV && accumulate) {
       p_(y.x);
@@ -1106,6 +1138,7 @@ struct Pass2SFT : NoStreams, Pass2SFRhs<FV> {
       if (k.use_lower) p_.n(S_YZL, y.zl);
       if (k.use_upper) p_.n(S_YZU, y.zu);
     }
+    if constexpr (HD) p_.n(S_H, this->h);
     for (int j = 0; j < ncols; j++) p_.n(S_V0 + j, V.p[j]);
     p_.w(W_CW, Cw); p_.w(W_D2, d2);
     p_.w(W_SW, v.sw); p_.w(W_TW, v.tw); p_.w(W_ZSW, v.zsw); p_.w(W_ZTW, v.ztw);
@@ -1262,6 +1295,12 @@ struct Pass2SFT : NoStreams, Pass2SFRhs<FV> {
     if (k.use_lower) stv<W>(y.zl, i, pzl);
     if (k.use_upper) stv<W>(y.zu, i, pzu);
     stats_elements<W>(k, tau, x, l, u, zl, zu, px, pzl, pzu, gv, acc);
+    if constexpr (HD) {
+      double hv[W];
+      src.template ld<W>(S_H, this->h, i, hv);
+#pragma unroll
+      for (int q = 0; q < W; q++) acc.s[22] = fma(hv[q] * px[q], px[q], acc.s[22]);
+    }
 #pragma unroll
     for (int q = 0; q < W; q++) {
       part2[q][0] = coef[q] * x[q];
@@ -1285,6 +1324,7 @@ struct Pass2SFT : NoStreams, Pass2SFRhs<FV> {
 // distinct types, so that kernel names and profiles tell the two passes apart
 struct Pass2SF : Pass2SFT<0> {};
 struct Pass2SVF : Pass2SFT<1> {};
+struct Pass2SVHF : Pass2SFT<1, 1> {};
 
 // ============================================================== TrialF
 // Line-search trial point (IP.cpp:3997-4013: rx, rsw, rtw via computeStepVec)

@@ -41,6 +41,11 @@ struct pcu_problem {
     return 1;
   }
   virtual bool hasHvecProduct() const { return false; }
+  // h = the diagonal of the Hessian of the Lagrangian at (x, z, zw); the optimizer calls
+  // it after every gradient evaluation when use_diag_hessian is set, and refuses that
+  // option for a problem without it.
+  virtual int evalHessianDiag(pcu_vec *, const double *, pcu_vec *, pcu_vec *) { return 1; }
+  virtual bool hasHessianDiag() const { return false; }
 };
 
 WDesc pcu_make_wdesc(const pcu_weighting &w, int nvars);

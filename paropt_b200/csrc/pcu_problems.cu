@@ -318,10 +318,43 @@ struct SQConGradF : NoStreams {  // A_j[i] = a_lo + a_w u(100 + j, gi), up to 8 
   }
 };
 
+// diag(P diag(lam) P) = lam - c1 v^2 lam + c2 v^2, c1 = 4 / (v.v), c2 = 4 (v.lam v) / (v.v)^2;
+// with vlam set the pass only reduces v.lam v (once per problem)
+struct SQHessDiagF : NoStreams {
+  static constexpr int NS = 1, NX = 0, NM = 0, NB = 0;
+  typedef Acc<NS, NX, NM> AccT;
+  typedef Con0 Con;
+  struct Elem {};
+  const double *lam, *vh;
+  double *h;
+  double c1, c2;
+  template <int W>
+  __device__ __forceinline__ void A(long long, const double (&)[W], Elem (&)[W],
+                                    double (&)[W][1], AccT *acc) const {}
+  __device__ __forceinline__ void B(long long, const double (&)[1], Con &,
+                                    AccT &) const {}
+  template <int W>
+  __device__ __forceinline__ void C(long long i, const double (&)[W],
+                                    const Elem (&)[W], const Con &,
+                                    AccT &acc) const {
+    double l[W], v[W], o[W];
+    ldv<W>(lam, i, l);
+    ldv<W>(vh, i, v);
+#pragma unroll
+    for (int e = 0; e < W; e++) {
+      const double v2 = v[e] * v[e];
+      if (h) o[e] = (l[e] - c1 * (v2 * l[e])) + c2 * v2;
+      else acc.s[0] = fma(v2, l[e], acc.s[0]);
+    }
+    if (h) stv<W>(h, i, o);
+  }
+};
+
 struct SepQuadProblem : pcu_problem {
   SepQuadDev q;
   pcu_vec *lam = nullptr, *b = nullptr, *vh = nullptr;
   double vtv = 0.0;
+  double vlv = -1.0;  // v^T diag(lam) v (Householder), reduced at the first evalHessianDiag
   std::vector<double> beta;
 
   ~SepQuadProblem() {
@@ -411,6 +444,33 @@ struct SepQuadProblem : pcu_problem {
     return grad_into(px, hvec, false);
   }
   bool hasHvecProduct() const override { return true; }
+
+  // The Hessian is constant (the constraints are linear): its exact diagonal, lam without
+  // the reflector, else the diagonal of P diag(lam) P.
+  int evalHessianDiag(pcu_vec *, const double *, pcu_vec *, pcu_vec *h) override {
+    if (!q.p.householder) return pcu_vec_copy(h, lam);
+    SQHessDiagF f;
+    f.lam = lam->d;
+    f.vh = vh->d;
+    if (vlv < 0.0) {
+      f.h = nullptr;
+      RedBuf rb = ctx->redbuf(1, 0, 0);
+      if (pcu_launch_tile(ctx, f, nvars, no_weighting(), rb)) return 1;
+      if (ctx->fetch(&vlv)) return 1;
+    }
+    f.h = h->d;
+    f.c1 = 4.0 / vtv;
+    f.c2 = 4.0 * vlv / (vtv * vtv);
+    RedBuf rb = ctx->redbuf(1, 0, 0);
+    if (pcu_launch_tile(ctx, f, nvars, no_weighting(), rb)) return 1;
+    // (no sum in this pass: drop its reduction slot without a host round trip)
+    if (!ctx->pending.empty()) {
+      ctx->result_used = ctx->pending.back().offset;
+      ctx->pending.pop_back();
+    }
+    return 0;
+  }
+  bool hasHessianDiag() const override { return true; }
 
   int evalObjConGradient(pcu_vec *x, pcu_vec *g, pcu_vec **Ac) override {
     if (grad_into(x, g, true)) return 1;
@@ -591,6 +651,13 @@ struct CallbackProblem : pcu_problem {
     return cb.eval_hvec_product ? cb.eval_hvec_product(cb.user, x, z, zw, px, hvec) : 1;
   }
   bool hasHvecProduct() const override { return cb.eval_hvec_product != nullptr; }
+  // pcu_problem_set_hessian_diag
+  void *hd_user = nullptr;
+  int (*hd_eval)(void *, pcu_vec *, const double *, pcu_vec *, pcu_vec *) = nullptr;
+  int evalHessianDiag(pcu_vec *x, const double *z, pcu_vec *zw, pcu_vec *h) override {
+    return hd_eval ? hd_eval(hd_user, x, z, zw, h) : 1;
+  }
+  bool hasHessianDiag() const override { return hd_eval != nullptr; }
 };
 
 // ======================================================= host-array callbacks
@@ -606,7 +673,12 @@ struct HostProblem : pcu_problem {
   double t_d2h = 0.0, t_user = 0.0, t_h2d = 0.0;  // wall-clock ms per phase
   bool timing = false;  // PCU_HOST_TIMING: synchronise after the uploads to time them
   double *hx = nullptr, *hg = nullptr, *hzw = nullptr;
+  double *hh = nullptr;  // the diagonal Hessian's mirror (allocated at its first call)
   std::vector<double *> hA;
+  // pcu_problem_set_hessian_diag_host
+  void *hd_user = nullptr;
+  int (*hd_eval)(void *, int, const double *, const double *, int, const double *,
+                 double *) = nullptr;
   cudaEvent_t up_done = nullptr;  // last host->device copy of g / A
   bool up_pending = false;
 
@@ -614,6 +686,7 @@ struct HostProblem : pcu_problem {
     if (hx) cudaFreeHost(hx);
     if (hg) cudaFreeHost(hg);
     if (hzw) cudaFreeHost(hzw);
+    if (hh) cudaFreeHost(hh);
     for (double *p : hA)
       if (p) cudaFreeHost(p);
     if (up_done) cudaEventDestroy(up_done);
@@ -723,6 +796,32 @@ struct HostProblem : pcu_problem {
     return fail;
   }
   bool hasHvecProduct() const override { return cb.eval_hvec_product != nullptr; }
+  // h = diag H(x, z, zw) on host arrays: x in hx, zw copied to the host, h in its own
+  // mirror and one host->device copy
+  int evalHessianDiag(pcu_vec *x, const double *z, pcu_vec *zw, pcu_vec *h) override {
+    if (!hd_eval) return 1;
+    if (fetch_x(x)) return 1;
+    if (nwcon > 0 && !hzw)
+      PCU_CUDA_OK(cudaHostAlloc(&hzw, sizeof(double) * (size_t)nwcon, cudaHostAllocDefault));
+    if (!hh)
+      PCU_CUDA_OK(cudaHostAlloc(&hh, sizeof(double) * (size_t)(nvars > 0 ? nvars : 1),
+                                cudaHostAllocDefault));
+    if (wait_uploads()) return 1;  // hh of the previous call may still be on its way
+    if (nwcon > 0) {
+      PCU_CUDA_OK(cudaMemcpyAsync(hzw, zw->d, sizeof(double) * (size_t)nwcon,
+                                  cudaMemcpyDeviceToHost, ctx->stream));
+      PCU_CUDA_OK(cudaStreamSynchronize(ctx->stream));
+      d2h_bytes += (long long)(sizeof(double) * (size_t)nwcon);
+    }
+    const double t0 = host_now_ms();
+    const int fail = hd_eval(hd_user, nvars, hx, z, nwcon, hzw, hh);
+    t_user += host_now_ms() - t0;
+    if (push(h, hh)) return 1;
+    PCU_CUDA_OK(cudaEventRecord(up_done, ctx->stream));
+    up_pending = true;
+    return fail;
+  }
+  bool hasHessianDiag() const override { return hd_eval != nullptr; }
 };
 
 extern "C" {
@@ -753,6 +852,30 @@ pcu_problem *pcu_problem_create(pcu_ctx *ctx, int nvars, int ncon,
 }
 
 void pcu_problem_destroy(pcu_problem *prob) { delete prob; }
+
+int pcu_problem_set_hessian_diag(pcu_problem *prob, void *user,
+                                 int (*eval_hessian_diag)(void *user, pcu_vec *x,
+                                                          const double *z, pcu_vec *zw,
+                                                          pcu_vec *h)) {
+  CallbackProblem *p = dynamic_cast<CallbackProblem *>(prob);
+  if (!p) return 1;
+  p->hd_user = user;
+  p->hd_eval = eval_hessian_diag;
+  return 0;
+}
+
+int pcu_problem_set_hessian_diag_host(pcu_problem *prob, void *user,
+                                      int (*eval_hessian_diag)(void *user, int n,
+                                                               const double *x,
+                                                               const double *z, int nw,
+                                                               const double *zw,
+                                                               double *h)) {
+  HostProblem *p = dynamic_cast<HostProblem *>(prob);
+  if (!p) return 1;
+  p->hd_user = user;
+  p->hd_eval = eval_hessian_diag;
+  return 0;
+}
 
 pcu_problem *pcu_problem_create_host(pcu_ctx *ctx, int nvars, int ncon,
                                      int ninequality, int nwinequality,

@@ -890,6 +890,10 @@ int pcu_tr_set_option_int(pcu_tr *tr, const char *name, int value) {
     fprintf(stderr, "paropt_b200: tr_use_soc is not built\n");
     return 1;
   }
+  if (k == "use_diag_hessian" && value != 0) {
+    fprintf(stderr, "ParOpt error: use_diag_hessian is not available in the trust region\n");
+    return 1;
+  }
   pending_of(tr).push_back({k, 1, 0.0, value, ""});
   (void)known;
   return 0;
