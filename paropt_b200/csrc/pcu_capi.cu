@@ -638,11 +638,11 @@ int pcu_ip_merit_init_deriv(pcu_ip *ip, double max_x, double *merit,
 }
 
 int pcu_ip_get_gram(pcu_ip *ip, double *G, double *Ce, int *q) {
-  if (G && !ip->Graw.empty())
-    memcpy(G, ip->Graw.data(), sizeof(double) * ip->Graw.size());
-  if (q) *q = (int)round(sqrt((double)ip->Ceraw.size()));
-  if (Ce && !ip->Ceraw.empty())
-    memcpy(Ce, ip->Ceraw.data(), sizeof(double) * ip->Ceraw.size());
+  const DenseOff &o = ip->dense_off;  // (all zero before the first setup)
+  const double *h = ip->dense_host;
+  if (q) *q = o.q;
+  if (G && h) memcpy(G, h + o.Graw, sizeof(double) * o.c * o.c);
+  if (Ce && h) memcpy(Ce, h + o.Ceraw, sizeof(double) * o.q * o.q);
   return 0;
 }
 

@@ -5,7 +5,10 @@
 // runs either on the device without a host round trip (pcu_dense.cu: single-CTA kernel
 // on a flat work buffer staged in shared memory) or, with the same statements, on the
 // host (pcu_dense_host).  The one iterative-refinement step of that solve is done here,
-// in the column space of V = [A|Z] (pcu_dense_solve).  Reference: setUpKKTDiagSystem's
+// in the column space of V = [A|Z] (pcu_dense_solve).  Every other route of the host
+// (pcu_ip::setUpKKTSystem, computeKKTStep, the GMRES preconditioner, the starting points,
+// the quasi-Newton M) calls the same functions, on any width up to PCU_MAX_COLS, and
+// keeps its factors in the same flat buffer.  Reference: setUpKKTDiagSystem's
 // G (IP.cpp:1932-1969, dgetrf), setUpKKTSystem's Ce (IP.cpp:2646-2664, dgetrf), the
 // dense part of solveKKTDiagSystem (IP.cpp:2150-2170, 2288-2306) and of computeKKTStep
 // (IP.cpp:2716-2735), computeKKTRes / addKKTResStep's dense residual
@@ -14,7 +17,7 @@
 //
 // The device replaces the divisions on its critical path by reciprocals (<= 1 ulp
 // each), so the device and host runs agree to round-off (tests/test_gpu_gram_paths.py
-// holds the two histories to 1e-12).
+// holds the two histories to 1e-12).  The host divides, as LAPACK does.
 #pragma once
 
 #include <cuda_runtime.h>
@@ -30,6 +33,7 @@
 
 // Offsets (in doubles) into the flat work buffer.  [0, S) is written by the host
 // before the chain (inputs), [S, total) is produced on the device and read back.
+// m <= PCU_DENSE_MAXM on the device; the host routes take up to PCU_MAX_COLS columns.
 struct DenseOff {
   int c, q, ld, m;
   int mu, vz, vs, vt, vzs, vzt, cc, gs, gt;  // inputs: barrier, dense variables, c(x), penalties
@@ -70,8 +74,9 @@ static inline DenseOff pcu_dense_offsets(int c, int q, int ld) {
   o.yz = take(c); o.ys = take(c); o.yt = take(c); o.yzs = take(c); o.yzt = take(c);
   o.r = take(o.m); o.vtp = take(o.m);
   p = (p + 1) & ~1;
-  o.coef = take(PCU_DENSE_MAXM);
-  o.alpha2 = take(PCU_DENSE_MAXM);
+  const int ncoef = o.m > PCU_DENSE_MAXM ? o.m : PCU_DENSE_MAXM;  // >= the constant bank
+  o.coef = take(ncoef);
+  o.alpha2 = take(ncoef);
   o.total = (p + 1) & ~1;
   return o;
 }
@@ -130,8 +135,9 @@ PCU_HDN double pcu_dense_div(double a, double b) {
 }
 
 // LAPACK dgetrf / dgetrs restated (partial pivoting, first largest entry, column-major;
-// n <= 32); pivots are kept as doubles inside the flat buffer, invd receives the
-// reciprocal diagonal.  Same elimination order as pcu_lu_factor / pcu_lu_solve of pcu_ip.cu.
+// n <= 32 on the device, any n on the host); pivots are kept as doubles inside the flat
+// buffer, invd receives the reciprocal diagonal.  The solves read invd on the device only
+// (the host divides by the diagonal and may pass NULL).
 PCU_HDN int pcu_dense_lu_factor(int n, double *A, double *piv, double *invd) {
   int info = 0;
 #pragma unroll 1
@@ -184,7 +190,9 @@ PCU_HDN int pcu_dense_lu_factor(int n, double *A, double *piv, double *invd) {
     if (PCU_LANE == 0) invd[k] = inv;
     PCU_PFOR(i, k + 1, n) A[i + n * k] *= inv;
     PCU_SYNC();
-    // trailing update: a lane owns row i (n <= 32), its multiplier stays in a register
+    // trailing update: a lane owns row i (n <= 32), its multiplier stays in a register;
+    // the host runs down the columns (the same operation on every element)
+#ifdef __CUDA_ARCH__
     PCU_PFOR(i, k + 1, n) {
       const double lik = A[i + n * k];
 #pragma unroll 1
@@ -193,6 +201,13 @@ PCU_HDN int pcu_dense_lu_factor(int n, double *A, double *piv, double *invd) {
         if (akj != 0.0) A[i + n * j] -= lik * akj;
       }
     }
+#else
+    for (int j = k + 1; j < n; j++) {
+      const double akj = A[k + n * j];
+      if (akj != 0.0)
+        for (int i = k + 1; i < n; i++) A[i + n * j] -= A[i + n * k] * akj;
+    }
+#endif
     PCU_SYNC();
   }
   return info;
@@ -222,7 +237,11 @@ PCU_HDN void pcu_dense_lu_solve(int n, const double *LU, const double *piv, cons
   }
 #pragma unroll 1
   for (int k = n - 1; k >= 0; k--) {
+#ifdef __CUDA_ARCH__
     if (PCU_LANE == 0) b[k] *= invd[k];
+#else
+    b[k] /= LU[k + n * k];
+#endif
     PCU_SYNC();
     const double bk = b[k];
     PCU_PFOR(i, 0, k) b[i] -= LU[i + n * k] * bk;
@@ -253,7 +272,11 @@ PCU_HDN void pcu_dense_lu_solve_lane(int n, const double *LU, const double *piv,
   }
 #pragma unroll 1
   for (int k = n - 1; k >= 0; k--) {
+#ifdef __CUDA_ARCH__
     b[k] *= invd[k];
+#else
+    b[k] /= LU[k + n * k];
+#endif
     const double bk = b[k];
 #pragma unroll 1
     for (int i = 0; i < k; i++) b[i] -= LU[i + n * k] * bk;
@@ -291,7 +314,7 @@ PCU_HDN void pcu_dense_residual(double *w, const DenseOff &o, int with_step) {
 }
 
 // G = C0 + S_AA, Ce = S_ZZ - S_ZA G^-1 S_AZ - M / (d d^T), both LU-factored
-// (the host statements of pcu_ip::setUpKKTSystem).  scratch: >= c * q doubles.
+// (IP.cpp:1932-1969, 2646-2664).  scratch: >= c * q doubles.
 PCU_HDN void pcu_dense_setup(double *w, const DenseOff &o, double *scratch) {
   const int c = o.c, q = o.q, ld = o.ld, m = o.m;
   double *S = w + o.S;

@@ -26,60 +26,6 @@ int pcu_gram_enqueue(pcu_ctx *ctx, const ColTable &cols, int m,
 
 static const RedBuf NO_RED = {nullptr, nullptr, nullptr, 0};
 
-// ------------------------------------------------------------ small dense LU
-// Same algorithm as LAPACK dgetrf/dgetrs (partial pivoting, column-major), used
-// for G (ncon x ncon, IP.cpp:1969), Ce (q x q, IP.cpp:2664) and the
-// quasi-Newton M (QN.cpp:375, 743).
-int pcu_lu_factor(int n, double *A, int *piv) {
-  int info = 0;
-  for (int k = 0; k < n; k++) {
-    int p = k;
-    double best = fabs(A[k + (size_t)n * k]);
-    for (int i = k + 1; i < n; i++) {
-      const double v = fabs(A[i + (size_t)n * k]);
-      if (v > best) {
-        best = v;
-        p = i;
-      }
-    }
-    piv[k] = p;
-    if (A[p + (size_t)n * k] == 0.0) {
-      if (!info) info = k + 1;
-      continue;
-    }
-    if (p != k) {
-      for (int j = 0; j < n; j++) std::swap(A[k + (size_t)n * j], A[p + (size_t)n * j]);
-    }
-    const double inv = 1.0 / A[k + (size_t)n * k];
-    for (int i = k + 1; i < n; i++) A[i + (size_t)n * k] *= inv;
-    for (int j = k + 1; j < n; j++) {
-      const double akj = A[k + (size_t)n * j];
-      if (akj != 0.0) {
-        for (int i = k + 1; i < n; i++)
-          A[i + (size_t)n * j] -= A[i + (size_t)n * k] * akj;
-      }
-    }
-  }
-  return info;
-}
-
-void pcu_lu_solve(int n, const double *LU, const int *piv, double *b) {
-  for (int k = 0; k < n; k++) {
-    if (piv[k] != k) std::swap(b[k], b[piv[k]]);
-  }
-  for (int k = 0; k < n; k++) {
-    const double bk = b[k];
-    if (bk != 0.0) {
-      for (int i = k + 1; i < n; i++) b[i] -= LU[i + (size_t)n * k] * bk;
-    }
-  }
-  for (int k = n - 1; k >= 0; k--) {
-    b[k] /= LU[k + (size_t)n * k];
-    const double bk = b[k];
-    for (int i = 0; i < k; i++) b[i] -= LU[i + (size_t)n * k] * bk;
-  }
-}
-
 // ============================================================== QuasiNewton
 QuasiNewton::~QuasiNewton() {
   for (auto v : S) pcu_vec_destroy(v);
@@ -154,7 +100,7 @@ void QuasiNewton::z_table(ColTable &t, int off) const {
 void QuasiNewton::solve_compact(const double *rz, double *kap) const {
   const int q = size();
   for (int i = 0; i < q; i++) kap[i] = rz[i] * d0[i];
-  if (q > 0) pcu_lu_solve(q, Mf.data(), piv.data(), kap);
+  if (q > 0) pcu_dense_lu_solve(q, Mf.data(), piv.data(), nullptr, kap);
   for (int i = 0; i < q; i++) kap[i] *= d0[i];
 }
 
@@ -210,8 +156,9 @@ void QuasiNewton::mat_update() {
     d0.assign(q, 1.0);
   }
   Mf = M;
-  piv.assign(size() > 0 ? size() : 1, 0);
-  if (size() > 0) pcu_lu_factor(size(), Mf.data(), piv.data());
+  piv.assign(size() > 0 ? size() : 1, 0.0);
+  std::vector<double> invd(piv.size());  // (read by the device's solves only)
+  if (size() > 0) pcu_dense_lu_factor(size(), Mf.data(), piv.data(), invd.data());
 }
 
 // ParOptLBFGS::update (QN.cpp:162-334) / ParOptLSR1::update (QN.cpp:636-747).

@@ -1,6 +1,7 @@
 // pcu_ip.cuh -- host-side interior-point driver (ParOptInteriorPoint mirror).
 #pragma once
 
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -96,7 +97,7 @@ struct QuasiNewton {
   std::vector<pcu_vec *> S, Y, Zs;
   pcu_vec *r = nullptr;
   std::vector<double> D, L, B, M, d0, Mf;
-  std::vector<int> piv;
+  std::vector<double> piv;  // pivots of Mf, as doubles (the dense buffer's format)
 
   ~QuasiNewton();
   int init(pcu_ctx *c, int nvars, int kind, int m);
@@ -165,11 +166,6 @@ struct pcu_ip {
   std::string qn_built_type;
   int qn_built_size = -1;
 
-  // dense factors
-  std::vector<double> Sgram;  // last Gram matrix (ld = sld), V = [A | Z]
-  int sld = 0, sq = 0;        // sq = quasi-Newton width used in the Gram
-  std::vector<double> Graw, Gfac, Ceraw, Cefac;
-  std::vector<int> gpiv, cpiv;
   double b0_used = 0.0;
 
   double barrier_param = 0.1, rho_penalty_search = 0.0;
@@ -200,8 +196,20 @@ struct pcu_ip {
   int opt_force_chain = 0;    // PCU_CHAIN=1: device chain also across GPUs
   int opt_no_gaz = 0;         // debugging (PCU_NO_GAZ): the update pass does not leave g - A z
   int opt_no_chain = 0;       // debugging (PCU_NO_CHAIN): dense algebra of the KKT solve on the host
-  double *dense_dev = nullptr, *dense_host = nullptr;  // work buffer of pcu_dense_kernel (+ pinned mirror)
+  // The dense state of the KKT solve (pcu_dense.cuh): its inputs, the Gram matrix of
+  // V = [A | Z], G and Ce with their LU factors.  dense_host (pinned) holds it in the
+  // layout dense_off of the last setUpKKTSystem / kktChain; dense_dev is the work buffer
+  // of pcu_dense_kernel.
+  DenseOff dense_off = DenseOff();
+  double *dense_dev = nullptr, *dense_host = nullptr;
   int dense_cap = 0;
+  int denseReserve(const DenseOff &o);
+  void densePack(const DenseOff &o, const Vars &vars, double mu, const double *gdiag);
+  // quasi-Newton columns of a solve with the factors of the last setup: that setup's, or
+  // none with use_qn = 0 or after a reset
+  int denseWidth(int use_qn) const {
+    return (qn && use_qn) ? std::min(dense_off.q, qn->size()) : 0;
+  }
   int pass1_ready = 0;        // Pass2R1F left d1', d2' and [A|Z]^T t1' for the next solve
   std::vector<double> pass1_r;
   double stats_pmax = 0.0;  // |px|_inf of the last StatsF launch

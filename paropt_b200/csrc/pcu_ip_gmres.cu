@@ -28,7 +28,6 @@
 
 int pcu_mdot_enqueue(pcu_ctx *ctx, const double *x, const ColTable &cols,
                      int ncols, long long n, int dst_off);
-void pcu_lu_solve(int n, const double *LU, const int *piv, double *b);
 
 #define launch_tile pcu_launch_tile
 static const RedBuf NO_RED = {nullptr, nullptr, nullptr, 0};
@@ -94,9 +93,12 @@ int pcu_ip::computeKKTGMRESStep(Vars &vars, Vars &res, Vars &step, double rtol,
     gmres_W.push_back(w);
   }
   std::vector<pcu_vec *> &W = gmres_W;
-  const int q = (qn && use_qn && !Cefac.empty()) ? std::min(sq, qn->size()) : 0;
+  const int q = denseWidth(use_qn);
   const int m = ncon + q;
-  const int ld = sld;
+  // the Gram matrix and the factors of the last setup
+  const DenseOff &o = dense_off;
+  const double *h = dense_host, *S = h + o.S;
+  const int ld = o.ld;
   const IPConst kc = kconst();
   ColTable V;
   for (int j = 0; j < ncon; j++) V.p[j] = Ac[j]->d;
@@ -230,7 +232,7 @@ int pcu_ip::computeKKTGMRESStep(Vars &vars, Vars &res, Vars &step, double rtol,
       yz1[j] = bs * (res.z[j] + (res.zs[j] + vars.s[j] * res.s[j]) / vars.zs[j] -
                      (res.zt[j] + vars.t[j] * res.t[j]) / vars.zt[j]) - r[j];
     }
-    if (ncon > 0) pcu_lu_solve(ncon, Gfac.data(), gpiv.data(), yz1.data());
+    if (ncon > 0) pcu_dense_lu_solve(ncon, h + o.Gfac, h + o.gpiv, h + o.ginv, yz1.data());
     for (int j = 0; j < ncon; j++) {
       step.z[j] = yz1[j];
       step.zs[j] = yz1[j] - bs * res.s[j];
@@ -260,16 +262,16 @@ int pcu_ip::computeKKTGMRESStep(Vars &vars, Vars &res, Vars &step, double rtol,
       // -G^-1 A^T D0^-1 Z w = -G^-1 S_AZ w (IP.cpp:5927-5945); only x is corrected
       for (int kq = 0; kq < q; kq++) {
         double v = r[ncon + kq];
-        for (int j = 0; j < ncon; j++) v += Sgram[(ncon + kq) + (size_t)ld * j] * yz1[j];
+        for (int j = 0; j < ncon; j++) v += S[(ncon + kq) + (size_t)ld * j] * yz1[j];
         wq[kq] = v;
       }
-      pcu_lu_solve(q, Cefac.data(), cpiv.data(), wq.data());
+      pcu_dense_lu_solve(q, h + o.Cefac, h + o.cpiv, h + o.ceinv, wq.data());
       for (int j = 0; j < ncon; j++) {
         double v = 0.0;
-        for (int kq = 0; kq < q; kq++) v += Sgram[j + (size_t)ld * (ncon + kq)] * wq[kq];
+        for (int kq = 0; kq < q; kq++) v += S[j + (size_t)ld * (ncon + kq)] * wq[kq];
         yz2[j] = -v;
       }
-      if (ncon > 0) pcu_lu_solve(ncon, Gfac.data(), gpiv.data(), yz2.data());
+      if (ncon > 0) pcu_dense_lu_solve(ncon, h + o.Gfac, h + o.gpiv, h + o.ginv, yz2.data());
       Pass2F f3 = f2;
       f3.y = refine.dv();
       f3.ncols = m;
@@ -279,13 +281,13 @@ int pcu_ip::computeKKTGMRESStep(Vars &vars, Vars &res, Vars &step, double rtol,
       std::swap(step.v[PCU_X], refine.v[PCU_X]);
       for (int j = 0; j < ncon; j++) {
         double v = r[j];
-        for (int jj = 0; jj < m; jj++) v += Sgram[j + (size_t)ld * jj] * f3.alpha.v[jj];
+        for (int jj = 0; jj < m; jj++) v += S[j + (size_t)ld * jj] * f3.alpha.v[jj];
         ATp[j] = v;
       }
     } else {
       for (int j = 0; j < ncon; j++) {
         double v = r[j];
-        for (int jj = 0; jj < ncon; jj++) v += Sgram[j + (size_t)ld * jj] * yz1[jj];
+        for (int jj = 0; jj < ncon; jj++) v += S[j + (size_t)ld * jj] * yz1[jj];
         ATp[j] = v;
       }
     }

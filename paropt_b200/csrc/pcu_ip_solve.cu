@@ -14,8 +14,6 @@ int pcu_gram_enqueue(pcu_ctx *ctx, const ColTable &cols, int m,
                      const double *Dinv, const double *Cw, const WDesc &wd,
                      long long n, int *ld_out, const double *d2 = nullptr,
                      int rhs_col = -1);
-int pcu_lu_factor(int n, double *A, int *piv);
-void pcu_lu_solve(int n, const double *LU, const int *piv, double *b);
 
 #define launch_tile pcu_launch_tile
 static const RedBuf NO_RED = {nullptr, nullptr, nullptr, 0};
@@ -104,12 +102,11 @@ int pcu_ip::setUpKKTDiagRhs(Vars &vars, int use_qn, double mu) {
 // One weighted Gram pass S = [A|Z]^T D0^-1 [A|Z] gives
 //   G  = C0 + S_AA                                  (IP.cpp:1932-1969)
 //   Ce = S_ZZ - S_ZA G^-1 S_AZ - M / (d d^T)        (IP.cpp:2646-2664)
-// gdiag: diagonal added to G (s/zs + t/zt, or `small` for the least-squares
-// start); NULL means s/zs + t/zt of `vars`.
+// (pcu_dense_setup, into dense_host).  gdiag: diagonal added to G (s/zs + t/zt, or
+// `small` for the least-squares start); NULL means s/zs + t/zt of `vars`.
 int pcu_ip::setUpKKTSystem(Vars &vars, int use_qn, const double *gdiag,
                            int with_rhs) {
   const int q = (qn && use_qn) ? qn->size() : 0;
-  sq = q;
   const int m = ncon + q;
   ColTable V;
   for (int j = 0; j < ncon; j++) V.p[j] = Ac[j]->d;
@@ -124,52 +121,66 @@ int pcu_ip::setUpKKTSystem(Vars &vars, int use_qn, const double *gdiag,
     } else {
       if (pcu_gram_enqueue(ctx, V, m, Dinv->d, Cw->d, wd, nvars, &ld)) return 1;
     }
-    Sgram.assign((size_t)ld * ld, 0.0);
-    if (ctx->big_fetch((size_t)ld * ld, Sgram.data())) return 1;
+  }
+  const DenseOff o = pcu_dense_offsets(ncon, q, ld);
+  if (denseReserve(o)) return 1;
+  dense_off = o;
+  double *h = dense_host;
+  if (m > 0) {
+    if (ctx->big_fetch((size_t)ld * ld, h + o.S)) return 1;
     if (with_rhs) {
       pass1_r.resize(m);
-      for (int j = 0; j < m; j++) pass1_r[j] = Sgram[m + (size_t)ld * j];
+      for (int j = 0; j < m; j++) pass1_r[j] = h[o.S + m + (size_t)ld * j];
       pass1_ready = 1;
     }
-    for (int j = 0; j < m; j++)  // symmetrise from the lower triangle
-      for (int i = j + 1; i < m; i++)
-        Sgram[j + (size_t)ld * i] = Sgram[i + (size_t)ld * j];
   }
-  sld = ld;
-  Graw.assign((size_t)ncon * ncon, 0.0);
-  for (int j = 0; j < ncon; j++)
-    for (int i = 0; i < ncon; i++) Graw[i + (size_t)ncon * j] = Sgram[i + (size_t)ld * j];
-  for (int i = 0; i < ncon; i++) {
-    Graw[i * (size_t)(ncon + 1)] +=
-        gdiag ? gdiag[i] : vars.s[i] / vars.zs[i] + vars.t[i] / vars.zt[i];
-  }
-  Gfac = Graw;
-  gpiv.assign(ncon > 0 ? ncon : 1, 0);
-  if (ncon > 0) pcu_lu_factor(ncon, Gfac.data(), gpiv.data());
-  Ceraw.clear();
-  Cefac.clear();
-  if (q > 0) {
-    Ceraw.assign((size_t)q * q, 0.0);
-    std::vector<double> col(ncon);
-    for (int i = 0; i < q; i++) {
-      // column i: Z^T P Z_i - S_ZA G^-1 (A^T P Z_i)
-      for (int j = 0; j < ncon; j++) col[j] = Sgram[j + (size_t)ld * (ncon + i)];
-      if (ncon > 0) pcu_lu_solve(ncon, Gfac.data(), gpiv.data(), col.data());
-      for (int k = 0; k < q; k++) {
-        double v = Sgram[(ncon + k) + (size_t)ld * (ncon + i)];
-        for (int j = 0; j < ncon; j++) v -= Sgram[(ncon + k) + (size_t)ld * j] * col[j];
-        Ceraw[k + (size_t)q * i] = v;
-      }
-    }
-    const std::vector<double> &M = qn->M, &d0 = qn->d0;
-    for (int j = 0; j < q; j++)
-      for (int i = 0; i < q; i++)
-        Ceraw[i + (size_t)q * j] -= M[i + (size_t)q * j] / (d0[i] * d0[j]);
-    Cefac = Ceraw;
-    cpiv.assign(q, 0);
-    pcu_lu_factor(q, Cefac.data(), cpiv.data());
-  }
+  densePack(o, vars, barrier_param, gdiag);
+  std::vector<double> scratch(PCU_DENSE_SCRATCH(ncon, q));
+  pcu_dense_setup(h, o, scratch.data());
   return 0;
+}
+
+// dense_host large enough for the layout `o` (its contents are lost when it grows).  It is
+// sized once for the widest solve the quasi-Newton object allows.  dense_dev follows it:
+// kktChain allocates it again when the device runs the dense algebra.
+int pcu_ip::denseReserve(const DenseOff &o) {
+  if (dense_host && dense_cap >= o.total) return 0;
+  if (dense_dev) cudaFree(dense_dev);
+  if (dense_host) cudaFreeHost(dense_host);
+  dense_dev = nullptr;
+  dense_host = nullptr;
+  const int qmax = qn ? qn->max_size() : 0;
+  dense_cap = pcu_dense_offsets(ncon, qmax, 8 * ((ncon + qmax + 1 + 7) / 8)).total + 64;
+  if (dense_cap < o.total) dense_cap = o.total + 64;
+  PCU_CUDA_OK(cudaMallocHost(&dense_host, sizeof(double) * dense_cap));
+  return 0;
+}
+
+// The inputs of the dense algebra at `vars` into dense_host, laid out by `o`.  gdiag (the
+// least-squares start's G = gdiag I + A^T D0^-1 A) is packed as s = gdiag, zs = 1, t = 0,
+// zt = 1: pcu_dense_setup's s/zs + t/zt is then gdiag exactly, and nothing else of that
+// setup reads the dense inputs.
+void pcu_ip::densePack(const DenseOff &o, const Vars &vars, double mu, const double *gdiag) {
+  double *h = dense_host;
+  h[o.mu] = mu;
+  h[o.mu + 1] = 0.0;
+  for (int i = 0; i < ncon; i++) {
+    h[o.vz + i] = vars.z[i];
+    h[o.vs + i] = gdiag ? gdiag[i] : vars.s[i];
+    h[o.vt + i] = gdiag ? 0.0 : vars.t[i];
+    h[o.vzs + i] = gdiag ? 1.0 : vars.zs[i];
+    h[o.vzt + i] = gdiag ? 1.0 : vars.zt[i];
+    h[o.cc + i] = c[i];
+    h[o.gs + i] = gamma_s[i];
+    h[o.gt + i] = gamma_t[i];
+  }
+  const int q = o.q;
+  if (q > 0) {
+    memcpy(h + o.M, qn->M.data(), sizeof(double) * q * q);
+    memcpy(h + o.d0, qn->d0.data(), sizeof(double) * q);
+    memcpy(h + o.Mf, qn->Mf.data(), sizeof(double) * q * q);
+    memcpy(h + o.mpiv, qn->piv.data(), sizeof(double) * q);
+  }
 }
 
 // ------------------------------------------------------------ computeKKTStep
@@ -185,7 +196,7 @@ int pcu_ip::computeKKTStep(Vars &vars, Vars &b, Vars &y, int use_qn,
   {
     // The residual-free first solve needs the fused pass-1 / pass-2 kernels;
     // otherwise materialise the right-hand side first.
-    const int q0 = (qn && use_qn && !Cefac.empty()) ? std::min(sq, qn->size()) : 0;
+    const int q0 = denseWidth(use_qn);
     // more than 32 columns: only with this solve's first half already done by the
     // Gram pass (pass 2 is then Pass2RF, which takes any width)
     const bool fused_ok = emit_res && VTp && !force_direct_dots &&
@@ -197,7 +208,8 @@ int pcu_ip::computeKKTStep(Vars &vars, Vars &b, Vars &y, int use_qn,
     }
     if (rhs_from_vars) denseResidual(vars, mu_res, b, nullptr, nullptr);
   }
-  const int q = (qn && use_qn && !Cefac.empty()) ? std::min(sq, qn->size()) : 0;
+  if (!dense_host) return 1;  // no setup yet
+  const int q = denseWidth(use_qn);
   const int m = ncon + q;
   const IPConst k = kconst();
   ColTable V;
@@ -287,64 +299,41 @@ int pcu_ip::computeKKTStep(Vars &vars, Vars &b, Vars &y, int use_qn,
       if (ctx->big_fetch(m, r.data())) return 1;
     }
   }
-  // dense solves (IP.cpp:2150-2170, 2716-2722, 2288-2306)
-  std::vector<double> yz1(ncon), pz(ncon), ps(ncon), pt(ncon), pzs(ncon), pzt(ncon);
+  // dense solves (IP.cpp:2150-2170, 2716-2722, 2288-2306): pcu_dense_step with the
+  // factors of the last setup, at this solve's width
+  DenseOff o = dense_off;
+  o.q = q;
+  o.m = m;
+  double *h = dense_host;
+  densePack(o, vars, mu_res, nullptr);
   for (int i = 0; i < ncon; i++) {
-    yz1[i] = (b.z[i] + (b.zs[i] + vars.s[i] * b.s[i]) / vars.zs[i] -
-              (b.zt[i] + vars.t[i] * b.t[i]) / vars.zt[i] - r[i]);
-  }
-  if (ncon > 0) pcu_lu_solve(ncon, Gfac.data(), gpiv.data(), yz1.data());
-  for (int i = 0; i < ncon; i++) {
-    pz[i] = yz1[i];
-    pzs[i] = yz1[i] - b.s[i];
-    pzt[i] = -b.t[i] - yz1[i];
-    ps[i] = (b.zs[i] - vars.s[i] * pzs[i]) / vars.zs[i];
-    pt[i] = (b.zt[i] - vars.t[i] * pzt[i]) / vars.zt[i];
-  }
-  Pass2F f2;
-  for (int i = 0; i < ncon; i++) f2.alpha.v[i] = yz1[i];
-  if (q > 0) {
-    const int ld = sld;
-    std::vector<double> w(q), yz2(ncon);
-    for (int kq = 0; kq < q; kq++) {  // Z^T yx = r_Z + S_ZA yz1
-      double v = r[ncon + kq];
-      for (int j = 0; j < ncon; j++) v += Sgram[(ncon + kq) + (size_t)ld * j] * yz1[j];
-      w[kq] = v;
-    }
-    pcu_lu_solve(q, Cefac.data(), cpiv.data(), w.data());
-    for (int j = 0; j < ncon; j++) {  // second solve: A^T P Z w = S_AZ w
-      double v = 0.0;
-      for (int kq = 0; kq < q; kq++) v += Sgram[j + (size_t)ld * (ncon + kq)] * w[kq];
-      yz2[j] = -v;
-    }
-    if (ncon > 0) pcu_lu_solve(ncon, Gfac.data(), gpiv.data(), yz2.data());
-    for (int i = 0; i < ncon; i++) {
-      const double yzs2 = yz2[i], yzt2 = -yz2[i];
-      const double ys2 = -(vars.s[i] * yzs2) / vars.zs[i];
-      const double yt2 = -(vars.t[i] * yzt2) / vars.zt[i];
-      pz[i] -= yz2[i];
-      pzs[i] -= yzs2;
-      pzt[i] -= yzt2;
-      ps[i] -= ys2;
-      pt[i] -= yt2;
-      f2.alpha.v[i] = pz[i];
-    }
-    for (int kq = 0; kq < q; kq++) f2.alpha.v[ncon + kq] = -w[kq];
-  }
-  for (int i = 0; i < ncon; i++) {
+    h[o.bz + i] = b.z[i];
+    h[o.bs + i] = b.s[i];
+    h[o.bt + i] = b.t[i];
+    h[o.bzs + i] = b.zs[i];
+    h[o.bzt + i] = b.zt[i];
     if (accumulate) {
-      y.z[i] += pz[i];
-      y.s[i] += ps[i];
-      y.t[i] += pt[i];
-      y.zs[i] += pzs[i];
-      y.zt[i] += pzt[i];
-    } else {
-      y.z[i] = pz[i];
-      y.s[i] = ps[i];
-      y.t[i] = pt[i];
-      y.zs[i] = pzs[i];
-      y.zt[i] = pzt[i];
+      h[o.yz + i] = y.z[i];
+      h[o.ys + i] = y.s[i];
+      h[o.yt + i] = y.t[i];
+      h[o.yzs + i] = y.zs[i];
+      h[o.yzt + i] = y.zt[i];
     }
+  }
+  for (int i = 0; i < m; i++) {
+    h[o.r + i] = r[i];
+    h[o.vtp + i] = accumulate && VTp ? VTp[i] : 0.0;
+  }
+  std::vector<double> scratch(PCU_DENSE_SCRATCH(ncon, q));
+  pcu_dense_step(h, o, accumulate, h + o.coef, scratch.data());
+  Pass2F f2;
+  for (int j = 0; j < m; j++) f2.alpha.v[j] = h[o.coef + j];
+  for (int i = 0; i < ncon; i++) {
+    y.z[i] = h[o.yz + i];
+    y.s[i] = h[o.ys + i];
+    y.t[i] = h[o.yt + i];
+    y.zs[i] = h[o.yzs + i];
+    y.zt[i] = h[o.yzt + i];
   }
   f2.v = vars.dv();
   f2.b = b.dv();
@@ -360,17 +349,12 @@ int pcu_ip::computeKKTStep(Vars &vars, Vars &b, Vars &y, int use_qn,
   f2.accumulate = accumulate;
   f2.k = k;
   // [A | Z]^T p.  When the Gram pass covered every quasi-Newton vector the
-  // products follow from linearity, [A|Z]^T D0^-1 (d1 + V alpha) = r + S alpha,
-  // without touching the N-vectors again.
+  // products follow from linearity, [A|Z]^T D0^-1 (d1 + V alpha) = r + S alpha
+  // (pcu_dense_step), without touching the N-vectors again.
   const int qa = qn ? qn->size() : 0;
   const bool derived = (q == qa) && !force_direct_dots;
-  if (VTp && derived) {
-    for (int i = 0; i < m; i++) {
-      double vv = r[i];
-      for (int j = 0; j < m; j++) vv += Sgram[i + (size_t)sld * j] * f2.alpha.v[j];
-      VTp[i] = accumulate ? VTp[i] + vv : vv;
-    }
-  }
+  if (VTp && derived)
+    for (int i = 0; i < m; i++) VTp[i] = h[o.vtp + i];
   if (emit_res && VTp && derived) {
     // pass 2 also writes the refinement residual (computeKKTRes +
     // addKKTResStep at the accumulated step) into `b`
@@ -532,41 +516,17 @@ int pcu_ip::kktChain(Vars &vars, Vars &b, Vars &y, int use_qn, double mu, double
   const int q = (qn && use_qn) ? qn->size() : 0;
   const int m = ncon + q;
   if (m < 1 || m > PCU_DENSE_MAXM) return 1;
-  sq = q;
   stats_ready = 0;
   pass1_ready = 0;
   if (setUpKKTDiagRhs(vars, use_qn, mu)) return 1;
   // ---- inputs of the dense algebra (1-7 KB)
   const int ld = 8 * ((m + 1 + 7) / 8);
   const DenseOff o = pcu_dense_offsets(ncon, q, ld);
-  if (!dense_host || dense_cap < o.total) {
-    if (dense_dev) cudaFree(dense_dev);
-    if (dense_host) cudaFreeHost(dense_host);
-    dense_dev = nullptr;
-    dense_cap = pcu_dense_offsets(ncon, qn ? qn->max_size() : 0, 40).total + 64;
-    if (dense_cap < o.total) dense_cap = o.total + 64;
-    PCU_CUDA_OK(cudaMallocHost(&dense_host, sizeof(double) * dense_cap));
-  }
+  if (denseReserve(o)) return 1;
   if (on_device && !dense_dev) PCU_CUDA_OK(cudaMalloc(&dense_dev, sizeof(double) * dense_cap));
+  dense_off = o;
   double *h = dense_host;
-  h[o.mu] = mu;
-  h[o.mu + 1] = 0.0;
-  for (int i = 0; i < ncon; i++) {
-    h[o.vz + i] = vars.z[i];
-    h[o.vs + i] = vars.s[i];
-    h[o.vt + i] = vars.t[i];
-    h[o.vzs + i] = vars.zs[i];
-    h[o.vzt + i] = vars.zt[i];
-    h[o.cc + i] = c[i];
-    h[o.gs + i] = gamma_s[i];
-    h[o.gt + i] = gamma_t[i];
-  }
-  if (q > 0) {
-    memcpy(h + o.M, qn->M.data(), sizeof(double) * q * q);
-    memcpy(h + o.d0, qn->d0.data(), sizeof(double) * q);
-    memcpy(h + o.Mf, qn->Mf.data(), sizeof(double) * q * q);
-    for (int i = 0; i < q; i++) h[o.mpiv + i] = (double)qn->piv[i];
-  }
+  densePack(o, vars, mu, nullptr);
   if (on_device)
     PCU_CUDA_OK(cudaMemcpyAsync(dense_dev, h, sizeof(double) * o.S, cudaMemcpyHostToDevice,
                                 ctx->stream));
@@ -653,16 +613,6 @@ int pcu_ip::kktChain(Vars &vars, Vars &b, Vars &y, int use_qn, double mu, double
     b.zt[i] = h[o.bzt + i];
   }
   for (int i = 0; i < m; i++) VTp[i] = h[o.vtp + i];
-  sld = ld;
-  Sgram.assign(h + o.S, h + o.S + (size_t)ld * ld);
-  Graw.assign(h + o.Graw, h + o.Graw + (size_t)ncon * ncon);
-  Gfac.assign(h + o.Gfac, h + o.Gfac + (size_t)ncon * ncon);
-  gpiv.assign(ncon > 0 ? ncon : 1, 0);
-  for (int i = 0; i < ncon; i++) gpiv[i] = (int)h[o.gpiv + i];
-  Ceraw.assign(h + o.Ceraw, h + o.Ceraw + (size_t)q * q);
-  Cefac.assign(h + o.Cefac, h + o.Cefac + (size_t)q * q);
-  cpiv.assign(q, 0);
-  for (int i = 0; i < q; i++) cpiv[i] = (int)h[o.cpiv + i];
   return 0;
 }
 
@@ -865,7 +815,9 @@ int pcu_ip::initLeastSquaresMultipliers() {
       if (pcu_mdot_enqueue(ctx, t1->d, V, ncon, nvars, 0)) return 1;
       if (ctx->big_fetch(ncon, z.data())) return 1;
       for (int i = 0; i < ncon; i++) z[i] = -z[i];
-      pcu_lu_solve(ncon, Gfac.data(), gpiv.data(), z.data());
+      const double *h = dense_host;
+      const DenseOff &o = dense_off;
+      pcu_dense_lu_solve(ncon, h + o.Gfac, h + o.gpiv, h + o.ginv, z.data());
     }
     Pass2F f2;
     for (int i = 0; i < ncon; i++) f2.alpha.v[i] = z[i];
