@@ -168,13 +168,7 @@ void QuasiNewton::mat_update() {
 // own s_qn / y_qn): the new pair is stored by exchanging buffers with the slot it
 // replaces instead of two N-sized copies (4 N words per iteration).
 static int qn_store(pcu_vec *slot, pcu_vec *src, int steal) {
-  if (steal && slot->owns && src->owns && slot->managed == src->managed && slot->n == src->n &&
-      slot->ctx == src->ctx) {
-    std::swap(slot->d, src->d);
-    std::swap(slot->host_touched, src->host_touched);
-    return 0;
-  }
-  return pcu_vec_copy(slot, src);
+  return steal ? pcu_vec_take(slot, src) : pcu_vec_copy(slot, src);
 }
 
 int QuasiNewton::update(pcu_vec *s, pcu_vec *y, double yTy, double yTs,
@@ -343,8 +337,8 @@ pcu_ip::~pcu_ip() {
   Vars *all[4] = {&variables, &residual, &update, &refine};
   for (auto vs : all)
     for (int i = 0; i < 8; i++) pcu_vec_destroy(vs->v[i]);
-  pcu_vec *single[] = {lb, ub, g, Dinv, Cw, d1, d2, t1, s_qn, y_qn, rx, rsw, rtw, gaz, apz1, apz2,
-                       hdiag};
+  pcu_vec *single[] = {lb, ub, g, Dinv, Cw, d1, d2, t1, s_qn, y_qn, rx, rsw, rtw, rzl, rzu, rzw,
+                       rzsw, rztw, gaz, apz1, apz2, hdiag};
   for (auto v : single) pcu_vec_destroy(v);
   for (auto v : Ac) pcu_vec_destroy(v);
   for (auto v : gmres_W) pcu_vec_destroy(v);
@@ -385,6 +379,7 @@ int pcu_ip::init(pcu_problem *p) {  // constructor, IP.cpp:182-438
   if (getenv("PCU_NO_CHAIN")) opt_no_chain = 1;
   if (getenv("PCU_CHAIN")) opt_force_chain = 1;
   if (getenv("PCU_NO_UPDSTATS")) opt_no_updstats = 1;
+  if (getenv("PCU_NO_TRIALUPD")) opt_no_trialupd = 1;
   if (getenv("PCU_NO_GAZ")) opt_no_gaz = 1;
   Vars *all[4] = {&variables, &residual, &update, &refine};
   for (auto vs : all) {

@@ -64,6 +64,19 @@ struct IPOptions {
   std::string problem_name;
 };
 
+// dst takes src's values; src's values are undefined afterwards.  Two vectors of the
+// optimizer's own exchange their buffers (no copy), so that every handle keeps its
+// identity; anything else is copied.
+static inline int pcu_vec_take(pcu_vec *dst, pcu_vec *src) {
+  if (dst->owns && src->owns && dst->managed == src->managed && dst->n == src->n &&
+      dst->ctx == src->ctx) {
+    std::swap(dst->d, src->d);
+    std::swap(dst->host_touched, src->host_touched);
+    return 0;
+  }
+  return pcu_vec_copy(dst, src);
+}
+
 struct Vars {  // ParOptVars (IP.h:373-389)
   pcu_vec *v[8] = {nullptr, nullptr, nullptr, nullptr,
                    nullptr, nullptr, nullptr, nullptr};
@@ -142,6 +155,8 @@ struct pcu_ip {
   pcu_vec *d1 = nullptr, *d2 = nullptr, *t1 = nullptr;  // KKT-solve scratch
   pcu_vec *s_qn = nullptr, *y_qn = nullptr;
   pcu_vec *rx = nullptr, *rsw = nullptr, *rtw = nullptr;  // line-search trial
+  // the multipliers of a first trial taken by TrialUpdateF (created on its first use)
+  pcu_vec *rzl = nullptr, *rzu = nullptr, *rzw = nullptr, *rzsw = nullptr, *rztw = nullptr;
   pcu_vec *hdiag = nullptr;  // use_diag_hessian: h of the last gradient evaluation
   // g - A z at the current point, written by the last update pass (ncon >= 3): the first
   // pass of the next KKT solve reads it instead of g and the ncon constraint gradients
@@ -192,6 +207,7 @@ struct pcu_ip {
   double upd_sums[11], upd_max[5], upd_min[2];
   int upd_stats_valid = 0;
   int opt_no_updstats = 0;    // debugging (PCU_NO_UPDSTATS): always run the residual pass
+  int opt_no_trialupd = 0;    // debugging (PCU_NO_TRIALUPD): first trial by TrialF, then Update1FT
   int checkpoint_failed = 0;
   int opt_force_chain = 0;    // PCU_CHAIN=1: device chain also across GPUs
   int opt_no_gaz = 0;         // debugging (PCU_NO_GAZ): the update pass does not leave g - A z
@@ -223,6 +239,9 @@ struct pcu_ip {
     double dm0_prev = 0.0, res_norm_prev = 0.0;
     int no_merit_function_improvement = 0, line_search_test = 0,
         line_search_failed = 0;
+    // the last line search rejected its first trial: the next one takes it with TrialF
+    // instead of the update pass, whose work would be lost again
+    int first_trial_rejected = 0;
     std::string info;
     double last_pnorm2 = 0.0;
   } ls;

@@ -1631,11 +1631,52 @@ int pcu_ip::iterate_once(int *converged) {
   int line_search_skipped = 0;
   ls.no_merit_function_improvement = 0;
 
+  // The first pass of computeStepAndUpdate (IP.cpp:4178-4216) from the step scaled by
+  // ax, az; z_new: the new dense multipliers
+  const bool form_pair = qn && uq;
+  auto launch_update1 = [&](auto f1, double ax, double az, const double *z_new) -> int {
+    f1.v = v.dv();
+    f1.p = upd.dv();
+    f1.lb = lb->d;
+    f1.ub = ub->d;
+    f1.g = g->d;
+    f1.ncon = ncon;
+    for (int j = 0; j < ncon; j++) {
+      f1.Acol.p[j] = Ac[j]->d;
+      f1.z.v[j] = z_new[j];
+    }
+    f1.yqn = form_pair ? y_qn->d : nullptr;
+    if (form_pair && gaz_valid && apz_state == 3 && apz1 && apz2) {
+      // -(g - A z+) = -(g - A z) + az A p_z: g - A z was left by the last update pass,
+      // A p_z by the two pass-2 kernels of this iteration's solves -- three vectors
+      // instead of g and the ncon constraint gradients
+      f1.g = gaz->d;
+      f1.ncon = 2;
+      f1.Acol.p[0] = apz1->d;
+      f1.Acol.p[1] = apz2->d;
+      f1.z.v[0] = az;
+      f1.z.v[1] = az;
+    }
+    f1.ax = ax;
+    f1.az = az;
+    f1.k = kconst();
+    if (decltype(f1)::NS > 0) {
+      RedBuf rb = ctx->redbuf(decltype(f1)::NS, decltype(f1)::NX, decltype(f1)::NM);
+      if (launch_tile(ctx, f1, nvars, wd, rb)) return 1;
+      ctx->defer();  // fetched together with Update2F's dots (or a callback's sums)
+      return 0;
+    }
+    return launch_tile(ctx, f1, nvars, wd, NO_RED);
+  };
+  // The line search's first trial ran as TrialUpdateF and was accepted: the update pass
+  // is done, its results wait in the trial buffers, and the next iteration's residual
+  // statistics (Update1FT<1>'s, fetched with the merit sums) in trial_u1.
+  int trial_updated = 0;
+  double trial_u1[9];
+
   // computeStepAndUpdate (IP.cpp:4169-4267)
   auto step_and_update = [&](double a, int eval_obj_con) -> int {
     const double ax = a * alpha_x, az = a * alpha_z;
-    const bool form_pair = qn && uq;
-    const IPConst kc = kconst();
     for (int i = 0; i < ncon; i++) {  // dense parts (IP.cpp:4190-4194)
       const double dp = opt.design_precision;
       auto clip0 = [&](double x0, double st, double p) {
@@ -1654,41 +1695,20 @@ int pcu_ip::iterate_once(int *converged) {
     // at the new point (Update1FT<1> / Update2FT<1>): its stand-alone residual pass
     // and one synchronisation disappear.
     const bool take_stats = form_pair && lazy_res && norm_type_id() == 0 && !opt_no_updstats;
-    auto launch_update1 = [&](auto f1) -> int {
-      f1.v = v.dv();
-      f1.p = upd.dv();
-      f1.lb = lb->d;
-      f1.ub = ub->d;
-      f1.g = g->d;
-      f1.ncon = ncon;
-      for (int j = 0; j < ncon; j++) {
-        f1.Acol.p[j] = Ac[j]->d;
-        f1.z.v[j] = v.z[j];
-      }
-      f1.yqn = form_pair ? y_qn->d : nullptr;
-      if (form_pair && gaz_valid && apz_state == 3 && apz1 && apz2) {
-        // -(g - A z+) = -(g - A z) + az A p_z: g - A z was left by the last update pass,
-        // A p_z by the two pass-2 kernels of this iteration's solves -- three vectors
-        // instead of g and the ncon constraint gradients
-        f1.g = gaz->d;
-        f1.ncon = 2;
-        f1.Acol.p[0] = apz1->d;
-        f1.Acol.p[1] = apz2->d;
-        f1.z.v[0] = az;
-        f1.z.v[1] = az;
-      }
-      f1.ax = ax;
-      f1.az = az;
-      f1.k = kc;
-      if (decltype(f1)::NS > 0) {
-        RedBuf rb = ctx->redbuf(decltype(f1)::NS, decltype(f1)::NX, decltype(f1)::NM);
-        if (launch_tile(ctx, f1, nvars, wd, rb)) return 1;
-        ctx->defer();  // fetched together with Update2F's dots (or a callback's sums)
-        return 0;
-      }
-      return launch_tile(ctx, f1, nvars, wd, NO_RED);
-    };
-    if (take_stats ? launch_update1(Update1FT<1>()) : launch_update1(Update1FT<0>())) return 1;
+    if (trial_updated) {
+      // the trial buffers become the variables (exchanged: the handles keep their
+      // identity); the bound multipliers only where the pass wrote them
+      if (pcu_vec_take(v.v[PCU_X], rx) ||
+          (prob->use_lower && pcu_vec_take(v.v[PCU_ZL], rzl)) ||
+          (prob->use_upper && pcu_vec_take(v.v[PCU_ZU], rzu)) ||
+          pcu_vec_take(v.v[PCU_ZW], rzw) || pcu_vec_take(v.v[PCU_SW], rsw) ||
+          pcu_vec_take(v.v[PCU_TW], rtw) || pcu_vec_take(v.v[PCU_ZSW], rzsw) ||
+          pcu_vec_take(v.v[PCU_ZTW], rztw))
+        return 1;
+    } else if (take_stats ? launch_update1(Update1FT<1>(), ax, az, v.z.data())
+                          : launch_update1(Update1FT<0>(), ax, az, v.z.data())) {
+      return 1;
+    }
     if (eval_obj_con) {
       if (evalObjCon(v.v[PCU_X])) {
         fprintf(stderr, "ParOpt: Function and constraint evaluation failed\n");
@@ -1736,7 +1756,8 @@ int pcu_ip::iterate_once(int *converged) {
           if (decltype(f2)::NX > 0) {
             // residual statistics of the next iteration, in ResF's layout
             double u1[9];
-            if (ctx->take_deferred(u1, 9)) return 1;
+            if (trial_updated) memcpy(u1, trial_u1, sizeof(u1));
+            else if (ctx->take_deferred(u1, 9)) return 1;
             memset(upd_sums, 0, sizeof(upd_sums));
             upd_sums[0] = u1[0];
             upd_sums[1] = u1[1];
@@ -1791,25 +1812,58 @@ int pcu_ip::iterate_once(int *converged) {
     const int max_iters = opt.max_line_iters;
     std::vector<double> rs(ncon), rt(ncon);
     const double dp = opt.design_precision;
-    auto eval_trial = [&](double a, bool merit_too, double *merit_out) -> int {
-      TrialF ft;
-      ft.v = v.dv();
-      ft.p = upd.dv();
-      ft.lb = lb->d;
-      ft.ub = ub->d;
-      ft.rx = rx->d;
-      ft.rsw = rsw->d;
-      ft.rtw = rtw->d;
-      ft.ax = a * alpha_x;
-      ft.k = kconst();
-      RedBuf rb = ctx->redbuf(TrialF::NS, 0, 0);
-      if (launch_tile(ctx, ft, nvars, wd, rb)) return -1;
+    // update: the trial is the update pass (TrialUpdateF), in case it is accepted
+    auto eval_trial = [&](double a, bool merit_too, double *merit_out, bool update) -> int {
+      if (update) {
+        // spares of the multipliers the pass writes: 3W, and N per bound in use
+        pcu_vec **wv[] = {&rzw, &rzsw, &rztw};
+        for (auto pv : wv)
+          if (!*pv && !(*pv = pcu_vec_create(ctx, nwcon))) return -1;
+        if (prob->use_lower && !rzl && !(rzl = pcu_vec_create(ctx, nvars))) return -1;
+        if (prob->use_upper && !rzu && !(rzu = pcu_vec_create(ctx, nvars))) return -1;
+        TrialUpdateF fu;
+        fu.r.x = rx->d;
+        fu.r.zl = rzl ? rzl->d : nullptr;
+        fu.r.zu = rzu ? rzu->d : nullptr;
+        fu.r.zw = rzw->d;
+        fu.r.sw = rsw->d;
+        fu.r.tw = rtw->d;
+        fu.r.zsw = rzsw->d;
+        fu.r.ztw = rztw->d;
+        const double az = a * alpha_z;
+        std::vector<double> z_new(ncon);
+        for (int i = 0; i < ncon; i++) z_new[i] = v.z[i] + az * upd.z[i];
+        if (launch_update1(fu, a * alpha_x, az, z_new.data())) return -1;
+      } else {
+        TrialF ft;
+        ft.v = v.dv();
+        ft.p = upd.dv();
+        ft.lb = lb->d;
+        ft.ub = ub->d;
+        ft.rx = rx->d;
+        ft.rsw = rsw->d;
+        ft.rtw = rtw->d;
+        ft.ax = a * alpha_x;
+        ft.k = kconst();
+        RedBuf rb = ctx->redbuf(TrialF::NS, 0, 0);
+        if (launch_tile(ctx, ft, nvars, wd, rb)) return -1;
+        // the merit sums travel with the reductions the objective callback fetches
+        // (one synchronisation for both)
+        ctx->defer();
+      }
       double ts[TrialF::NS];
-      // the merit sums travel with the reductions the objective callback fetches
-      // (one synchronisation for both)
-      ctx->defer();
       int fail_obj = evalObjCon(rx);
-      if (ctx->take_deferred(ts, TrialF::NS)) return -1;
+      if (update) {
+        constexpr int TS = TrialUpdateF::TS, NS = TrialUpdateF::NS;
+        double all[NS + TrialUpdateF::NX + TrialUpdateF::NM];
+        if (ctx->take_deferred(all, NS + TrialUpdateF::NX + TrialUpdateF::NM)) return -1;
+        for (int i = 0; i < TrialF::NS; i++) ts[i] = all[TS + i];
+        // Update1FT<1>'s layout: its sums, then the maxima and minima
+        for (int i = 0; i < TS; i++) trial_u1[i] = all[i];
+        for (int i = 0; i < 9 - TS; i++) trial_u1[TS + i] = all[NS + i];
+      } else if (ctx->take_deferred(ts, TrialF::NS)) {
+        return -1;
+      }
       if (fail_obj) return 1;
       if (!merit_too) return 0;
       for (int i = 0; i < ncon; i++) {
@@ -1838,9 +1892,13 @@ int pcu_ip::iterate_once(int *converged) {
       *merit_out = m;
       return 0;
     };
+    // the first trial is also the update pass unless the last line search rejected
+    // its first trial
+    const bool update_first = !opt_no_trialupd && !ls.first_trial_rejected;
     int j = 0;
     for (; j < max_iters; j++) {
-      int rc = eval_trial(alpha, true, &merit);
+      int rc = eval_trial(alpha, true, &merit, j == 0 && update_first);
+      if (j == 0) ls.first_trial_rejected = 1;  // until the test below accepts it
       if (rc < 0) return -1;
       if (rc > 0) {
         fprintf(stderr,
@@ -1856,6 +1914,10 @@ int pcu_ip::iterate_once(int *converged) {
         if (fail & LS_MIN_STEP) fail = LS_SUCCESS | LS_MIN_STEP;
         else fail = LS_SUCCESS;
         if (merit <= m0 + fp && merit + fp >= m0) fail |= LS_NO_IMPROVEMENT;
+        if (j == 0) {
+          ls.first_trial_rejected = 0;
+          trial_updated = update_first;
+        }
         break;
       } else if (fail & LS_MIN_STEP) {
         break;
@@ -1892,7 +1954,7 @@ int pcu_ip::iterate_once(int *converged) {
       if (alpha != best_alpha) {
         alpha = best_alpha;
         double dummy;
-        int rc = eval_trial(alpha, false, &dummy);
+        int rc = eval_trial(alpha, false, &dummy, false);
         if (rc != 0) {
           fprintf(stderr, "ParOpt: Evaluation failed during line search\n");
           fail = LS_FAILURE;

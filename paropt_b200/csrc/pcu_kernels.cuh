@@ -1326,6 +1326,40 @@ struct Pass2SF : Pass2SFT<0> {};
 struct Pass2SVF : Pass2SFT<1> {};
 struct Pass2SVHF : Pass2SFT<1, 1> {};
 
+// The merit terms of a trial point, shared by TrialF and TrialUpdateF so that both
+// take them with the same expressions.  Slots from `o`: o, o+1 running product of the
+// bound barrier factors; o+2, o+3 that of sw tw; o+4 gam.(sw, tw); o+5 |cw - sw + tw|^2.
+// Barrier factor of one element at the trial point r.
+__device__ __forceinline__ double trial_bound_factor(const IPConst &k, double r, double l,
+                                                     double u) {
+  const bool ml = k.use_lower && l > -k.mbv;
+  const bool mu_ = k.use_upper && u < k.mbv;
+  const double dl = r - l, du = u - r;
+  return (ml ? dl : 1.0) * (mu_ ? du : 1.0);
+}
+template <int W, class AT>
+__device__ __forceinline__ void trial_bound_logs(int o, const double (&f)[W], AT &acc) {
+  if (W == 2) lp_mul2(acc.s[o], acc.s[o + 1], f[0], f[W - 1]);
+  else lp_mul(acc.s[o], acc.s[o + 1], f[0]);
+}
+// sw, tw: the trial slacks; sum0: the constraint's block sum of the trial point
+template <class AT>
+__device__ __forceinline__ void trial_constraint(int o, const IPConst &k, long long ci,
+                                                 double sw, double tw, double sum0,
+                                                 AT &acc) {
+  lp_mul(acc.s[o + 2], acc.s[o + 3], sw * tw);
+  acc.s[o + 4] += gamma_sw(k, ci) * sw + k.gamma * tw;
+  const double rw = ((wconst_at(k, ci) + sum0) - sw) + tw;
+  acc.s[o + 5] = fma(rw, rw, acc.s[o + 5]);
+}
+template <class AT>
+__device__ __forceinline__ void trial_finalize(int o, AT &acc) {
+  acc.s[o] = lp_value(acc.s[o], acc.s[o + 1]);
+  acc.s[o + 1] = 0.0;
+  acc.s[o + 2] = lp_value(acc.s[o + 2], acc.s[o + 3]);
+  acc.s[o + 3] = 0.0;
+}
+
 // ============================================================== TrialF
 // Line-search trial point (IP.cpp:3997-4013: rx, rsw, rtw via computeStepVec)
 // fused with the reductions of evalMeritFunc / evalInfeas (IP.cpp:3524-3601,
@@ -1372,11 +1406,8 @@ struct TrialF : NoStreams {
 #pragma unroll
     for (int q = 0; q < W; q++) {
       r[q] = step_clip(x[q], ax, px[q], l[q], u[q], k.dp);
-      const bool ml = k.use_lower && l[q] > -k.mbv;
-      const bool mu_ = k.use_upper && u[q] < k.mbv;
-      const double dl = r[q] - l[q], du = u[q] - r[q];
       // factor of the running product whose logarithm is the barrier sum
-      e[q].f = (ml ? dl : 1.0) * (mu_ ? du : 1.0);
+      e[q].f = trial_bound_factor(k, r[q], l[q], u[q]);
       part[q][0] = coef[q] * r[q];
     }
     stv<W>(rx, i, r);
@@ -1388,24 +1419,20 @@ struct TrialF : NoStreams {
     const double t = step_clip0(src.ldw(W_TW, v.tw, ci), ax, src.ldw(W_PTW, p.tw, ci), k.dp);
     rsw[ci] = s;
     rtw[ci] = t;
-    lp_mul(acc.s[2], acc.s[3], s * t);
-    acc.s[4] += gamma_sw(k, ci) * s + k.gamma * t;
-    const double rw = ((wconst_at(k, ci) + sum[0]) - s) + t;
-    acc.s[5] = fma(rw, rw, acc.s[5]);
+    trial_constraint(0, k, ci, s, t, sum[0], acc);
   }
   template <int W, class S, class AT>
   __device__ __forceinline__ void C(const S &, long long, const double (&)[W],
                                     const Elem (&e)[W], const Con &,
                                     AT &acc) const {
-    if (W == 2) lp_mul2(acc.s[0], acc.s[1], e[0].f, e[W - 1].f);
-    else lp_mul(acc.s[0], acc.s[1], e[0].f);
+    double f[W];
+#pragma unroll
+    for (int q = 0; q < W; q++) f[q] = e[q].f;
+    trial_bound_logs<W>(0, f, acc);
   }
   template <class AT>
   __device__ __forceinline__ void finalize(AT &acc) const {
-    acc.s[0] = lp_value(acc.s[0], acc.s[1]);
-    acc.s[1] = 0.0;
-    acc.s[2] = lp_value(acc.s[2], acc.s[3]);
-    acc.s[3] = 0.0;
+    trial_finalize(0, acc);
   }
 };
 
@@ -1422,12 +1449,26 @@ struct TrialF : NoStreams {
 // order as ResF.   sums: 0 bound comp product, 1 comp count, 2 sparse comp product;
 // maxima: 0 |rzw|, 1 |rsw| / |rtw|, 2 bound products, 3 sparse products; minima: 0
 // bound products, 1 sparse products.
-template <int STATS>
-struct Update1FT : NoStreams {
+// TRIAL = 1 (TrialUpdateF) runs BEFORE the objective callback as the line search's
+// first trial: the new point goes to r (r.x = rx, r.sw = rsw, r.tw = rtw: the trial
+// point TrialF would have written, bit for bit) instead of v, and the pass also takes
+// TrialF's six merit sums at it, in slots 3-8 (TrialF's 0-5).  The host exchanges r
+// with v when the trial is accepted -- one pass instead of TrialF + Update1FT.
+// Traffic: the words of Update1FT (TrialF's 5N + 6W disappear); six more sums, and the
+// merit terms' arithmetic on every element and constraint.
+template <int TRIAL> struct Update1Out { DVars r; };
+template <> struct Update1Out<0> {};
+template <int STATS, int TRIAL = 0>
+struct Update1FT : NoStreams, Update1Out<TRIAL> {
   static constexpr int SRC = 1;
-  static constexpr int REVERSE = 1;  // after TrialF and the objective callback (upwards)
-  static constexpr int NS = STATS ? 3 : 0, NX = STATS ? 4 : 0, NM = STATS ? 2 : 0,
-                       NB = STATS ? 1 : 0;
+  // from the last tile down: after TrialF, or with TRIAL after Pass2SVF, both of which
+  // walk from the first tile up
+  static constexpr int REVERSE = 1;
+  // the merit sums do not fit the register-fed kernel's 73 registers without spills
+  static constexpr int MINB = TRIAL ? 5 : NoStreams::MINB;
+  static constexpr int TS = STATS ? 3 : 0;  // first slot of the merit sums (TRIAL)
+  static constexpr int NS = TS + (TRIAL ? 6 : 0), NX = STATS ? 4 : 0,
+                       NM = STATS ? 2 : 0, NB = (STATS || TRIAL) ? 1 : 0;
   enum { S_X, S_PX, S_LB, S_UB, S_ZL, S_PZL, S_ZU, S_PZU, S_G, S_A0 };
   static constexpr int NFIX = S_A0;  // fixed slots; the columns follow
   static constexpr int TROWS = 512;
@@ -1459,6 +1500,11 @@ struct Update1FT : NoStreams {
   double *yqn;  // null when no quasi-Newton pair is formed
   double ax, az;
   IPConst k;
+
+  __device__ __forceinline__ const DVars &out() const {  // where the new point goes
+    if constexpr (TRIAL) return this->r;
+    else return v;
+  }
 
   template <class P>
   __device__ __forceinline__ void streams(P &p_) const {
@@ -1494,11 +1540,13 @@ struct Update1FT : NoStreams {
     const double tw = step_clip0(src.ldw(W_TW, v.tw, ci), ax, src.ldw(W_PTW, p.tw, ci), k.dp);
     const double zsw = step_clip0(src.ldw(W_ZSW, v.zsw, ci), az, src.ldw(W_PZSW, p.zsw, ci), k.dp);
     const double ztw = step_clip0(src.ldw(W_ZTW, v.ztw, ci), az, src.ldw(W_PZTW, p.ztw, ci), k.dp);
-    v.zw[ci] = zwn;
-    v.sw[ci] = sw;
-    v.tw[ci] = tw;
-    v.zsw[ci] = zsw;
-    v.ztw[ci] = ztw;
+    const DVars &o = out();
+    o.zw[ci] = zwn;
+    o.sw[ci] = sw;
+    o.tw[ci] = tw;
+    o.zsw[ci] = zsw;
+    o.ztw[ci] = ztw;
+    if (TRIAL) trial_constraint(TS, k, ci, sw, tw, sum[0], acc);  // TrialF::B
     if (STATS) {  // ResF::B at the new point
       const double gsw = gamma_sw(k, ci), gtw = k.gamma;
       const double rzw = -(((wconst_at(k, ci) + sum[0]) - sw) + tw);
@@ -1523,17 +1571,18 @@ struct Update1FT : NoStreams {
       x[q] = e[q].x;
       zl[q] = zu[q] = 0.0;
     }
-    if (STATS) {
+    if (STATS || TRIAL) {
       src.template ld<W>(S_LB, lb, i, l);
       src.template ld<W>(S_UB, ub, i, u);
     }
+    const DVars &o = out();
     if (k.use_lower) {
       double pzl[W];
       src.template ld<W>(S_ZL, v.zl, i, zl);
       src.template ld<W>(S_PZL, p.zl, i, pzl);
 #pragma unroll
       for (int q = 0; q < W; q++) zl[q] = step_clip0(zl[q], az, pzl[q], k.dp);
-      stv<W>(v.zl, i, zl);
+      stv<W>(o.zl, i, zl);
     }
     if (k.use_upper) {
       double pzu[W];
@@ -1541,7 +1590,7 @@ struct Update1FT : NoStreams {
       src.template ld<W>(S_PZU, p.zu, i, pzu);
 #pragma unroll
       for (int q = 0; q < W; q++) zu[q] = step_clip0(zu[q], az, pzu[q], k.dp);
-      stv<W>(v.zu, i, zu);
+      stv<W>(o.zu, i, zu);
     }
     if (yqn) {
       double gv[W], yv[W];
@@ -1558,7 +1607,13 @@ struct Update1FT : NoStreams {
       for (int q = 0; q < W; q++) yv[q] = fma(coef[q], con.d[0], yv[q]);
       stv<W>(yqn, i, yv);
     }
-    stv<W>(v.x, i, x);
+    stv<W>(o.x, i, x);
+    if (TRIAL) {  // TrialF::A / C: the barrier factors of the bounds
+      double f[W];
+#pragma unroll
+      for (int q = 0; q < W; q++) f[q] = trial_bound_factor(k, x[q], l[q], u[q]);
+      trial_bound_logs<W>(TS, f, acc);
+    }
     if (STATS) {  // ResF::A / C at the new point: complementarity of the bounds
 #pragma unroll
       for (int q = 0; q < W; q++) {
@@ -1587,8 +1642,14 @@ struct Update1FT : NoStreams {
       }
     }
   }
+  template <class AT>
+  __device__ __forceinline__ void finalize(AT &acc) const {
+    if (TRIAL) trial_finalize(TS, acc);
+  }
 };
 typedef Update1FT<0> Update1F;
+// a distinct type, so that kernel names and profiles tell it from the stand-alone pass
+struct TrialUpdateF : Update1FT<1, 1> {};
 
 // ============================================================== Update2F
 // computeStepAndUpdate, second half (IP.cpp:4244-4256) after the new gradients:
